@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload jacobi5|jacobi_r2|jacobi_r3|hotspot|fdtd|convection_pt|conway]
-                    [--rows R --cols C --iterations I]
+                    [--rows R --cols C --iterations I] [--dump-outputs DIR]
 
 Metric (BASELINE.json / reference scripts/benchmark-common.jl:97-98): GCell-updates/s =
 rows * cols * n_iterations / time, one "update" being one full iteration (all sub-iterations).
@@ -15,6 +15,8 @@ iterations. Default workload at N=1: BASELINE.json configs[1], Jacobi 5-point fp
                stream the kernels are launched on, barrier + synchronize on both sides, max over ranks.
 `e2e`          the same step through the public Grid/StencilUpdate API starting from cells in pinned
                host memory (GridAccessor image): upload + update + download inside the timed region.
+               Its own step count (`e2e.steps`) is min(--steps, 3), and 1 for slabs moved chunk by
+               chunk: --steps sets the timed steps of `value`, not of `e2e`.
 `roofline`     HBM roofline of the fused sweep kernel: algorithmic bytes (2*sizeof(Cell)*n_sub per
                cell-iteration, the reference's own model) per launch / mean launch duration, against
                the measured copy bandwidth in MEASURED_PEAKS.json.
@@ -28,6 +30,11 @@ iterations. Default workload at N=1: BASELINE.json configs[1], Jacobi 5-point fp
                same process: HotSpot 16384^2 (strong-scaled at N > 1, plus weak), FDTD max_grid
                (strong), mantle convection 8192 x 65536 cells per GPU (weak).
 `--impl reference` times the reference's CPU implementation instead (same metric/config keys).
+`--dump-outputs DIR` after the timed steps of every workload measured, writes the cells its last
+               timed step returned as DIR/<name>.npy (one file per cell field, float32 or float64) so
+               that two builds run with the same arguments can be compared output for output.
+               Outputs too large for the 64 MB limit are sampled on rows x columns chosen with a
+               fixed seed (see `dump_sample`).
 
 Multi-GPU (torchrun, one rank per GPU): the grid is row-sharded, every rank owns `rows` rows (weak
 scaling) or a share of a fixed grid (strong), and exchanges halo rows with its neighbours once per
@@ -403,6 +410,52 @@ def check_parity_window(workload, params, halo, fill, total_rows, cols, iters, r
             "build": ("-fmad=false" if strict_build else "default (-fmad=true)") + ", the planner's plan"}
 
 
+# ---------------------------------------------------------------------------------------------------
+# --dump-outputs
+# ---------------------------------------------------------------------------------------------------
+
+DUMP_BYTES = 60 << 20   # all files of one invocation: under 64 MB with the .npy headers
+DUMP_SEED = 20240607
+
+
+def dump_dtype(field_dtype: np.dtype) -> np.dtype:
+    """float64 for 8-byte fields, float32 for everything narrower (Conway's bool cells included)."""
+    return np.dtype(np.float64) if field_dtype.itemsize == 8 else np.dtype(np.float32)
+
+
+def dump_sample(total_rows: int, cols: int, dtype: np.dtype, budget: int):
+    """(row indices, column indices) of the cells --dump-outputs writes: the whole grid where it fits
+    `budget` bytes, else a near-square sample of rows x columns. On each axis the sample holds both
+    ends (the cells that read the halo, and where e.g. convection's boundary temperatures start) and
+    a scatter of the rest drawn with a fixed seed. The choice depends only on its arguments, so every
+    run with the same command line dumps the same cells."""
+    fields = [dtype[name] for name in dtype.names] if dtype.names else [dtype]
+    cell_bytes = sum(dump_dtype(f).itemsize for f in fields)
+    cells = max(1, budget // cell_bytes)
+    if total_rows * cols <= cells:
+        return np.arange(total_rows), np.arange(cols)
+    n_rows = min(total_rows, max(1, int(np.sqrt(cells))))
+    n_cols = min(cols, max(1, cells // n_rows))
+    rng = np.random.default_rng(DUMP_SEED)
+
+    def pick(n_total, n_pick):
+        if n_pick >= n_total:
+            return np.arange(n_total)
+        edge = min(64, n_pick // 4)
+        scatter = rng.choice(np.arange(edge, n_total - edge), n_pick - 2 * edge, replace=False)
+        return np.sort(np.concatenate([np.arange(edge), np.arange(n_total - edge, n_total), scatter]))
+    return pick(total_rows, n_rows), pick(cols, n_cols)
+
+
+def write_dump(directory: Path, name: str, cells: np.ndarray) -> None:
+    """One .npy per cell field (`name.field.npy`), or `name.npy` for single-value cells."""
+    directory.mkdir(parents=True, exist_ok=True)
+    for field in (cells.dtype.names or (None,)):
+        values = cells[field] if field else cells
+        np.save(directory / (f"{name}.{field}.npy" if field else f"{name}.npy"),
+                np.ascontiguousarray(values, dtype=dump_dtype(values.dtype)))
+
+
 def workload_config(workload, total_rows, rows, cols, iters, world):
     """The `config` object; identical in both arms (it names the workload, not the implementation)."""
     return {
@@ -525,8 +578,9 @@ class Context:
             self.dist.destroy_process_group()
 
 
-def measure(args, ctx: Context, cpu_seconds: float = 12.0, parity: bool = True):
-    """One workload, measured as the module docstring says. Collective; rank 0 gets the record."""
+def measure(args, ctx: Context, cpu_seconds: float = 12.0, parity: bool = True, dump=None):
+    """One workload, measured as the module docstring says. Collective; rank 0 gets the record.
+    `dump` = (directory, name, byte budget): where --dump-outputs writes the last timed step's cells."""
     from stencilstream_b200 import Grid, Params, StencilUpdate, workload_info
     from stencilstream_b200 import _native
 
@@ -630,6 +684,21 @@ def measure(args, ctx: Context, cpu_seconds: float = 12.0, parity: bool = True):
         elapsed_ms = timer.end_ms()
         barrier()
     launches = n_launches() - launches_before
+    if dump is not None:
+        dump_dir, dump_name, dump_budget = dump
+        rows_idx, cols_idx = dump_sample(total_rows, cols, dtype, dump_budget)
+        if runner is None:
+            # Grid has no row-range download; the whole result is a temporary here, as it is for the
+            # end-to-end phase below, which downloads the same grid
+            sample = out.to_numpy()[np.ix_(rows_idx, cols_idx)]
+        else:   # only the sampled rows leave the device (a slab may be tens of GB)
+            mine = rows_idx[(rows_idx >= runner.row_lo) & (rows_idx < runner.row_hi)]
+            owned = np.empty((len(mine), cols), dtype=dtype)
+            for i, row in enumerate(mine):
+                runner.slab.copy_rows_to_host(int(row) - runner.row_lo, owned[i:i + 1])
+            sample = np.concatenate(ctx.gather(owned[:, cols_idx]))
+        if rank == 0:
+            write_dump(dump_dir, dump_name, sample)
     del out
     elapsed_ms = ctx.max_over_ranks(elapsed_ms)
 
@@ -702,7 +771,7 @@ def measure(args, ctx: Context, cpu_seconds: float = 12.0, parity: bool = True):
             # result grid and its pinned image alive: drop all of them before the next step allocates
             del mid, view, result
         e2e_value = total_cells * iters / float(np.mean(times)) / 1e9
-        e2e = {"value": e2e_value, "unit": "GCell-updates/s",
+        e2e = {"value": e2e_value, "unit": "GCell-updates/s", "steps": e2e_steps,
                "h2d_bytes_per_step": int(rows * cols * dtype.itemsize),
                "d2h_bytes_per_step": int(rows * cols * dtype.itemsize),
                "ms_per_step": float(np.mean(times) * 1e3), "checksum": checksum,
@@ -742,7 +811,7 @@ def measure(args, ctx: Context, cpu_seconds: float = 12.0, parity: bool = True):
         mid = host_out[min(rows // 2, host_out.shape[0] - 1), cols // 2]
         checksum = float(mid[dtype.names[0]] if dtype.names else mid)
         e2e = {"value": total_cells * iters / float(np.mean(times)) / 1e9, "unit": "GCell-updates/s",
-               "h2d_bytes_per_step": int(rows * cols * dtype.itemsize) * world,
+               "steps": e2e_steps, "h2d_bytes_per_step": int(rows * cols * dtype.itemsize) * world,
                "d2h_bytes_per_step": int(rows * cols * dtype.itemsize) * world,
                "ms_per_step": float(np.mean(times) * 1e3), "checksum": checksum,
                "host_memory": host_memory["kind"]}
@@ -804,21 +873,26 @@ SECONDARY = [
 ]
 
 
+def dump_target(args, name: str, budget: int):
+    return (Path(args.dump_outputs), name, budget) if args.dump_outputs else None
+
+
 def run_ours(args, ctx: Context, default_invocation: bool):
-    line = measure(args, ctx)
-    if default_invocation and not args.headline_only:
+    secondary = [s for s in SECONDARY if not (s[6] and ctx.world == 1)] \
+        if default_invocation and not args.headline_only else []
+    budget = DUMP_BYTES // (1 + len(secondary))
+    line = measure(args, ctx, dump=dump_target(args, args.workload, budget))
+    if secondary:
         import copy
         import gc
         workloads = {}
-        for key, workload, rows, cols, iters, scaling, multi_only in SECONDARY:
-            if multi_only and ctx.world == 1:
-                continue
+        for key, workload, rows, cols, iters, scaling, _ in secondary:
             sub = copy.copy(args)
             sub.workload, sub.rows, sub.cols, sub.iterations, sub.scaling = workload, rows, cols, iters, scaling
-            sub.steps, sub.warmup, sub.fuse = min(args.steps, 5), 3, 0
+            sub.fuse = 0
             gc.collect()
             try:
-                record = measure(sub, ctx, cpu_seconds=4.0)
+                record = measure(sub, ctx, cpu_seconds=4.0, dump=dump_target(args, key, budget))
             except Exception as exc:  # keep the headline line even if a secondary workload fails
                 record = {"error": f"{type(exc).__name__}: {exc}"[:300]}
             if ctx.rank == 0:
@@ -853,7 +927,13 @@ def main():
                     help="slabs larger than this many GiB are generated/transferred in row chunks")
     ap.add_argument("--no-overlap", action="store_true",
                     help="multi-GPU: one launch per pass instead of boundary-first scheduling")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the cells the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU implementation's outputs (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -877,7 +957,8 @@ def main():
         if default_invocation:
             run_ours(args, ctx, True)
         else:
-            line = measure(args, ctx, cpu_seconds=0.0 if args.no_cpu_baseline else 12.0)
+            line = measure(args, ctx, cpu_seconds=0.0 if args.no_cpu_baseline else 12.0,
+                           dump=dump_target(args, args.workload, DUMP_BYTES))
             if rank == 0:
                 print(json.dumps(line), flush=True)
     finally:

@@ -150,6 +150,50 @@ def load_golden(workload):
             "n_iterations": int(data["n_iterations"])}
 
 
+# ---- seeded cases checked against the reference build (tests/test_oracle.py) -----------------------
+# Their reference outputs travel with the repository as SHA-256 digests of the output bytes
+# (tests/golden/reference_digests.json), so the port is held to them where the reference tree is absent.
+
+SEEDED_SHAPES = [(1, 1), (5, 3), (37, 53)]
+WINDOW_SHAPE = (61, 67)
+
+
+def seeded_cases(workload, shape):
+    """[(key, params, halo, cells, iteration_offset, n_iterations)] of one workload and shape: seed 11,
+    (offset, n) = (0, 1) and (2, 4). Empty where the workload cannot be set up on that grid."""
+    if workload.startswith("convection") and min(shape) < 4:
+        return []   # the convection set-up needs at least a 4x4 grid (dx = lx / (nx - 1))
+    params, halo, cells = make_case(workload, *shape, seed=11)
+    out = []
+    for offset, n in ((0, 1), (2, 4)):
+        if "kat" in workload:
+            cells = kat_input(*shape, offset)
+        out.append((f"{workload} {shape[0]}x{shape[1]} seed=11 offset={offset} n={n}",
+                    params, halo, cells, offset, n))
+    return out
+
+
+def window_case(workload):
+    """(key, params, halo, cells, offset, n): the whole-grid run whose windows
+    test_window_oracle_equals_the_whole_grid_run crops (seed 3, offset 1, 3 iterations)."""
+    params, halo, cells = make_case(workload, *WINDOW_SHAPE, seed=3)
+    offset, n = 1, 3
+    if "kat" in workload:
+        cells = kat_input(*WINDOW_SHAPE, offset)
+    return (f"{workload} {WINDOW_SHAPE[0]}x{WINDOW_SHAPE[1]} seed=3 offset={offset} n={n}",
+            params, halo, cells, offset, n)
+
+
+def output_digest(cells):
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(cells).tobytes()).hexdigest()
+
+
+def load_reference_digests():
+    import json
+    return json.loads((GOLDEN_DIR / "reference_digests.json").read_text())["digests"]
+
+
 # ---- the convection application loop on the oracle (host-side glue as in the reference's main) ----------
 
 def oracle_convection(oracle, config):

@@ -15,6 +15,7 @@ They pin (a) the plain-C restatement oracle/stencil_oracle.c on machines without
 from __future__ import annotations
 
 import ctypes as C
+import json
 import sys
 from pathlib import Path
 
@@ -70,6 +71,22 @@ def main() -> None:
             n_iterations=np.array(n), seed=np.array(seed))
         print(f"{workload}: {cells.shape} offset={offset} n={n} -> {path.name} "
               f"({path.stat().st_size} bytes)")
+    write_reference_digests(ref, "SHA-256 of the output bytes of the reference build "
+                                 "(oracle/_ref/liboracle_ref.so), written by tests/golden/generate.py")
+
+
+def write_reference_digests(checker, provenance: str) -> None:
+    """tests/golden/reference_digests.json: the digest of `checker`'s output for every seeded case of
+    tests/test_oracle.py (cases.seeded_cases, cases.window_case)."""
+    digests = {}
+    for workload in cases.GOLDEN_WORKLOADS:
+        runs = [c for shape in cases.SEEDED_SHAPES for c in cases.seeded_cases(workload, shape)]
+        runs.append(cases.window_case(workload))
+        for key, params, halo, cells, offset, n in runs:
+            digests[key] = cases.output_digest(checker.run(workload, params, halo, cells, offset, n))
+    path = HERE / "reference_digests.json"
+    path.write_text(json.dumps({"provenance": provenance, "digests": digests}, indent=1) + "\n")
+    print(f"{len(digests)} digests -> {path.name}")
 
 
 if __name__ == "__main__":

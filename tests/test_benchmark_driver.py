@@ -126,6 +126,36 @@ def test_bench_parity_window_agrees_with_a_whole_grid_oracle_run(oracle_best, mo
         assert record["rel_max_norm"] <= 1e-5       # FMA vs two roundings after 12 iterations
 
 
+def test_bench_dump_sample_is_fixed_and_within_the_budget(tmp_path):
+    """--dump-outputs: the whole grid where it fits, else a seeded rows x columns sample that is the
+    same on every call; files are float32 (float64 for 8-byte fields) and stay under the budget."""
+    import numpy as np
+    from stencilstream_b200 import _native
+    bench = _bench()
+    rows, cols = bench.dump_sample(300, 200, _native.CELL_DTYPES["hotspot"], 1 << 20)
+    assert (rows == np.arange(300)).all() and (cols == np.arange(200)).all()
+    for workload in ("jacobi5", "hotspot", "fdtd", "convection_pt", "conway"):
+        dtype = _native.CELL_DTYPES[workload]
+        budget = bench.DUMP_BYTES // 4
+        rows, cols = bench.dump_sample(16384, 65536, dtype, budget)
+        again = bench.dump_sample(16384, 65536, dtype, budget)
+        assert (rows == again[0]).all() and (cols == again[1]).all()
+        assert len(set(rows)) == len(rows) and (np.diff(rows) > 0).all() and rows[-1] < 16384
+        assert (np.diff(cols) > 0).all() and cols[-1] < 65536
+        for picked, n in ((rows, 16384), (cols, 65536)):   # both borders of the grid are in it
+            assert picked[0] == 0 and picked[-1] == n - 1 and len(picked) < n
+        cells = np.zeros((len(rows), len(cols)), dtype=dtype)
+        bench.write_dump(tmp_path / workload, workload, cells)
+        files = sorted((tmp_path / workload).iterdir())
+        assert len(files) == max(1, len(dtype.names or ()))
+        assert sum(f.stat().st_size for f in files) <= budget + 128 * len(files)
+        for f in files:
+            assert np.load(f).dtype in (np.float32, np.float64)
+            assert np.load(f).shape == (len(rows), len(cols))
+    assert np.load(tmp_path / "convection_pt" / "convection_pt.T.npy").dtype == np.float64
+    assert np.load(tmp_path / "conway" / "conway.npy").dtype == np.float32
+
+
 NCU_CSV = '''==PROF== Connected to process 4242 (/usr/bin/python3.12)
 jacobi5 k=6 tile=43x240 call 0: 7.5 ms
 ==PROF== Profiling "fused_sweep_kernel" - 0: 0%....50%....100% - 9 passes

@@ -3,7 +3,9 @@
 The plain-C restatement (oracle/stencil_oracle.c) is pinned three ways:
   1. against the golden vectors in tests/golden/ (outputs of the reference's own cpu backend, built
      in place from /root/reference by tests/golden/generate.py) — bit for bit;
-  2. against the reference-built oracle (oracle/_ref) on further seeded cases, where that exists;
+  2. against the reference-built oracle (oracle/_ref) on further seeded cases, where that exists, and
+     everywhere against the reference's outputs of those cases stored as digests
+     (tests/golden/reference_digests.json);
   3. against the reference's own known-answer test: the self-checking functor of
      /root/reference/tests/TransFuncs.hpp:55-104 with the case matrix of
      tests/cpu/StencilUpdate.cpp:35-41 and tests/cuda/StencilUpdate.cpp:30-50, whose expected output is
@@ -35,17 +37,29 @@ def test_reference_build_reproduces_golden_vectors(workload, oracle_ref):
 
 
 @pytest.mark.parametrize("workload", cases.GOLDEN_WORKLOADS)
-@pytest.mark.parametrize("shape", [(1, 1), (5, 3), (37, 53)])
+@pytest.mark.parametrize("shape", cases.SEEDED_SHAPES)
 def test_port_matches_reference_build(workload, shape, oracle_port, oracle_ref):
-    if workload.startswith("convection") and min(shape) < 4:
+    if not cases.seeded_cases(workload, shape):
         pytest.skip("the convection set-up needs at least a 4x4 grid (dx = lx / (nx - 1))")
-    params, halo, cells = cases.make_case(workload, *shape, seed=11)
-    for offset, n in ((0, 1), (2, 4)):
-        if "kat" in workload:
-            cells = cases.kat_input(*shape, offset)
+    digests = cases.load_reference_digests()
+    for key, params, halo, cells, offset, n in cases.seeded_cases(workload, shape):
         a = oracle_port.run(workload, params, halo, cells, offset, n)
         b = oracle_ref.run(workload, params, halo, cells, offset, n)
-        assert a.tobytes() == b.tobytes(), (workload, shape, offset, n)
+        assert a.tobytes() == b.tobytes(), key
+        assert cases.output_digest(b) == digests[key], f"stored digest no longer the reference's: {key}"
+
+
+@pytest.mark.parametrize("workload", cases.GOLDEN_WORKLOADS)
+def test_port_reproduces_the_reference_digests(workload, oracle_port):
+    """The seeded cases of test_port_matches_reference_build and the whole-grid run of
+    test_window_oracle_equals_the_whole_grid_run, held against the reference build's outputs stored
+    as digests (tests/golden/reference_digests.json) — bit for bit, without the reference tree."""
+    digests = cases.load_reference_digests()
+    runs = [c for shape in cases.SEEDED_SHAPES for c in cases.seeded_cases(workload, shape)]
+    runs.append(cases.window_case(workload))
+    for key, params, halo, cells, offset, n in runs:
+        got = oracle_port.run(workload, params, halo, cells, offset, n)
+        assert cases.output_digest(got) == digests[key], key
 
 
 @pytest.mark.parametrize("case", REFERENCE_KAT_CASES)
@@ -118,16 +132,15 @@ WINDOWS = {  # of a 61 x 67 grid: corner, edge, interior, ragged corner, whole g
 def test_window_oracle_equals_the_whole_grid_run(workload, which, request):
     """Pins tests/window_oracle.py (the checker of the full-size GPU parity tests): the oracle run on
     the domain-of-dependence crop of a window — global coordinates through oracle_run_window2d — holds
-    bit for bit what the whole-grid run holds in that window."""
+    bit for bit what the whole-grid run holds in that window; the whole-grid run is the reference
+    build's (stored digest), so the windows are too."""
     import window_oracle
 
     oracle = request.getfixturevalue("oracle_port" if which == "port" else "oracle_ref")
-    shape = (61, 67)
-    params, halo, cells = cases.make_case(workload, *shape, seed=3)
-    offset, n = 1, 3
-    if "kat" in workload:
-        cells = cases.kat_input(*shape, offset)
+    shape = cases.WINDOW_SHAPE
+    key, params, halo, cells, offset, n = cases.window_case(workload)
     whole = oracle.run(workload, params, halo, cells, offset, n)
+    assert cases.output_digest(whole) == cases.load_reference_digests()[key], key
     for name, window in WINDOWS.items():
         got = window_oracle.expected_window(
             oracle, workload, params, halo, lambda r0, r1, c0, c1: cells[r0:r1, c0:c1], shape, window,

@@ -109,7 +109,7 @@ struct HotspotCell {
     static constexpr auto fields = std::make_tuple(&HotspotCell::temp, &HotspotCell::power);
     /// B200 extension (cuda/internal/Helpers.hpp): no HotSpot sweep ever changes the dissipated power.
     /// (The unmodified reference example has no such line and gets the same effect from the
-    /// run-time detection of StencilUpdate::run_speculative; FDTD below is left to that detection on
+    /// run-time detection of StencilUpdate::run_detected; FDTD below is left to that detection on
     /// purpose, so that both routes stay exercised.)
     static constexpr auto constant_fields = std::make_tuple(&HotspotCell::power);
 };

@@ -21,10 +21,11 @@
  *
  * What is different: instead of one launch per sweep, ceil(n_iterations / k) launches of the fused,
  * shared-memory-tiled kernel in cuda/internal/TileKernel.hpp, planned by cuda/internal/Planner.hpp.
- * Fields that a transition function only passes through (HotSpot's `power`, FDTD's material
- * coefficients) are detected at run time and no longer copied between the tile buffers — speculative
- * plane pass-through, verified by every launch and transparently repeated without the speculation if a
- * launch ever sees such a field change (see `run_speculative` below and run_tile in TileKernel.hpp).
+ * Fields that a transition function only passes through are no longer copied between the tile
+ * buffers (cuda/internal/PassThrough.hpp): declared by the cell type (HotSpot's `power`), or detected
+ * at run time (FDTD's material coefficients), verified by every launch and transparently repeated
+ * without them if a launch ever sees such a field change (see `run_detected` below and run_tile in
+ * TileKernel.hpp).
  * `split_cell_structure` is accepted for source compatibility; the device layout is decided by
  * `Grid<Cell>` from `Cell::fields` alone (planes whenever the cell lists its fields), so both
  * values select the same code path and produce the same results.
@@ -35,6 +36,7 @@
 #include "Grid.hpp"
 #include "internal/Helpers.hpp"
 #include "internal/Launch.hpp"
+#include "internal/PassThrough.hpp"
 #include "internal/Planner.hpp"
 #include "internal/Runtime.hpp"
 #include "internal/SlabUpdate.hpp"
@@ -59,8 +61,6 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
     using TDV = typename F::TimeDependentValue;
 
   private:
-    using Layout = internal::CellLayout<Cell>;
-
     static_assert(std::is_trivially_copyable_v<F>,
                   "transition functions are copied into kernel parameters and must be trivially "
                   "copyable");
@@ -127,21 +127,9 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
     StencilUpdate(StencilUpdate const &other)
         : params(other.params), n_processed_cells(other.n_processed_cells),
           walltime(other.walltime), n_launches(other.n_launches), last_plan(other.last_plan),
-          tensor_maps(), profile_events(other.profile_events), spec_probed(other.spec_probed),
-          n_spec_redos(other.n_spec_redos) {
-        // what was observed about the transition function travels with the copy; the device words
-        // (spec_flags) are per object and allocated on first use
-        for (unsigned q = 0; q < internal::max_spec_subiterations; q++)
-            spec_keep[q] = other.spec_keep[q];
-    }
+          tensor_maps(), profile_events(other.profile_events), pass_through(other.pass_through),
+          n_spec_redos(other.n_spec_redos) {}
     StencilUpdate &operator=(StencilUpdate const &) = delete;
-
-    ~StencilUpdate() {
-        if (spec_flags)
-            internal::device_free(spec_device, spec_flags, internal::default_stream(spec_device));
-        if (spec_host_flags)
-            internal::pinned_free(spec_host_flags);
-    }
 
     /**
      * Compute `n_iterations` iterations of the source grid and return the result as a new grid.
@@ -200,269 +188,12 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
     /// without being copied (speculative plane pass-through), and how many times an update had to
     /// be repeated because a launch saw such a plane change.
     unsigned get_passthrough_planes() const {
-        if (shards)
-            return shards->slabs.front()->passthrough_planes();
-        if (!spec_probed)
-            return 0;
-        unsigned m = all_planes;
-        for (unsigned q = 0; q < n_sub; q++)
-            m &= spec_keep[q];
-        return m;
+        return shards ? shards->slabs.front()->passthrough_planes() : pass_through.single_planes();
     }
     std::size_t get_n_speculation_redos() const { return n_spec_redos; }
 
   private:
-    static constexpr unsigned n_sub = unsigned(F::n_subiterations);
-    static constexpr unsigned all_planes =
-        Layout::n_planes >= 32 ? ~0u : ((1u << Layout::n_planes) - 1u);
-
-    static bool speculation_enabled() {
-        if constexpr (!internal::speculation_capable<F>())
-            return false;
-        static const bool enabled = internal::env_long("STST_SPECULATE", 1) != 0;
-        return enabled;
-    }
-
-    /// Planes of fields the cell type declares constant (`Cell::constant_fields`, see
-    /// cuda/internal/Helpers.hpp), if using them pays (same rule as for detected ones).
-    static constexpr unsigned declared_constant = internal::constant_fields_mask<Cell>();
-    static_assert(declared_constant != ~0u || Layout::n_planes >= 32,
-                  "every entry of Cell::constant_fields must also be listed in Cell::fields");
-
-    static bool declared_passthrough_pays() {
-        if constexpr (declared_constant == 0 || !internal::speculation_capable<F>()) {
-            return false;
-        } else {
-            std::size_t bytes = 0;
-            for (std::size_t i = 0; i < Layout::n_planes; i++)
-                if ((declared_constant >> i) & 1u)
-                    bytes += Layout::plane_bytes(i);
-            return speculation_enabled() && 4 * bytes >= sizeof(Cell) && sizeof(Cell) <= 64;
-        }
-    }
-
-    /**
-     * The generation loop with DECLARED constant fields: the pass-through kernels with a keep mask
-     * known at compile time. No observing launch and no read-back — the call stays asynchronous.
-     * With STST_VERIFY_CONSTANT_FIELDS=1 the kernels' own check of the kept planes is read after the
-     * last launch (one stream synchronisation) and a violated declaration throws std::logic_error.
-     */
-    GridImpl run_declared(GridImpl &source_grid) {
-        using namespace internal;
-        auto &source = source_grid.get_storage();
-        const unsigned grid_h = unsigned(source.height), grid_w = unsigned(source.width);
-        source.require_device();
-        if (spec_flags && spec_device != source.device) {
-            device_free(spec_device, spec_flags, default_stream(spec_device));
-            spec_flags = nullptr;
-        }
-        const std::size_t flag_bytes = sizeof(unsigned) * (max_spec_subiterations + 1);
-        if (!spec_flags) {
-            spec_device = source.device;
-            spec_flags = static_cast<unsigned *>(device_alloc(spec_device, flag_bytes, source.stream));
-            STST_RT_CHECK(stst_memset_async(spec_flags, 0, flag_bytes, source.stream));
-        }
-        Speculation spec{};
-        for (unsigned q = 0; q < n_sub; q++)
-            spec.keep[q] = spec_keep[q] = declared_constant & all_planes;
-        spec.flags = spec_flags;
-        spec_probed = true;
-        const LaunchPlan plan =
-            make_plan<F>(source.device, grid_h, grid_w, params.n_iterations, params.fused_iterations,
-                         params.tile_rows, spec.single_planes(n_sub, all_planes));
-        last_plan = plan;
-        GridImpl swap_a = source_grid.make_similar();
-        GridImpl swap_b = (params.n_iterations > plan.fused_iterations) ? source_grid.make_similar()
-                                                                         : swap_a;
-        swap_a.get_storage().allocate_device();
-        swap_b.get_storage().allocate_device();
-        GridImpl *pass_source = &source_grid, *pass_target = &swap_a;
-        std::size_t iteration = params.iteration_offset, remaining = params.n_iterations;
-        bool first = true;
-        while (remaining > 0) {
-            const unsigned n_gens = unsigned(std::min<std::size_t>(remaining, plan.fused_iterations));
-            launch(plan, pass_source->get_storage(), pass_target->get_storage(), iteration, n_gens,
-                   &spec);
-            iteration += n_gens;
-            remaining -= n_gens;
-            if (first) {
-                pass_source = &swap_a;
-                pass_target = &swap_b;
-                first = false;
-            } else {
-                std::swap(pass_source, pass_target);
-            }
-        }
-        pass_source->get_storage().device_written();
-        static const bool verify = env_long("STST_VERIFY_CONSTANT_FIELDS", 0) != 0;
-        if (verify) {
-            unsigned host_flags[max_spec_subiterations + 1] = {};
-            STST_RT_CHECK(stst_memcpy_d2h_async(host_flags, spec_flags, flag_bytes, source.stream));
-            STST_RT_CHECK(stst_stream_synchronize(source.stream));
-            if (host_flags[max_spec_subiterations] != 0)
-                throw std::logic_error(
-                    "StencilStream-B200: the transition function changed a field that its cell type "
-                    "lists in Cell::constant_fields (plane mask " +
-                    std::to_string(host_flags[max_spec_subiterations]) + ")");
-        }
-        return *pass_source;
-    }
-
-    /**
-     * The generation loop with speculative plane pass-through.
-     *
-     * The first launch this updater ever submits also *observes*: per sub-iteration, which planes
-     * came out of the transition function different from the centre cell that went in. Planes that
-     * never changed are from then on left in place by the tile sweeps instead of being copied from
-     * tile buffer to tile buffer, and planes untouched in every sub-iteration need only one tile
-     * buffer, so the tiles grow. Every launch still compares what the function returned for those
-     * planes with what went in (for a genuinely passed-through field the compiler folds that away)
-     * and reports any difference through a device flag, which is read when all launches of the call
-     * have been submitted. If a launch reports a difference — the field does change after all, e.g.
-     * FDTD's `hz_sum` once `iteration >= detect_iteration` — that plane is struck from the masks and
-     * the WHOLE call is repeated from the (never modified) source grid. The result is therefore
-     * always what the unspeculated loop computes; the price is that such calls end with a stream
-     * synchronisation even when `blocking` is false.
-     */
-    GridImpl run_speculative(GridImpl &source_grid) {
-        using namespace internal;
-        auto &source = source_grid.get_storage();
-        const unsigned grid_h = unsigned(source.height), grid_w = unsigned(source.width);
-        source.require_device();
-        if (spec_flags && spec_device != source.device) {
-            device_free(spec_device, spec_flags, default_stream(spec_device));
-            spec_flags = nullptr;
-        }
-        if (!spec_flags) {
-            spec_device = source.device;
-            spec_flags = static_cast<unsigned *>(
-                device_alloc(spec_device, sizeof(unsigned) * (max_spec_subiterations + 1),
-                             source.stream));
-        }
-        if (!spec_host_flags)
-            spec_host_flags = static_cast<unsigned *>(
-                pinned_alloc(sizeof(unsigned) * (max_spec_subiterations + 1)));
-        unsigned *host_flags = spec_host_flags;
-        // launches and profiling events of an attempt that is discarded must not be counted
-        const std::size_t launches_before = n_launches;
-        const std::size_t events_before = profile_events.size();
-        auto read_flags = [&] {
-            STST_RT_CHECK(stst_memcpy_d2h_async(host_flags, spec_flags,
-                                                sizeof(unsigned) * (max_spec_subiterations + 1),
-                                                source.stream));
-            STST_RT_CHECK(stst_stream_synchronize(source.stream));
-        };
-        auto clear_flags = [&] {
-            STST_RT_CHECK(stst_memset_async(spec_flags, 0,
-                                            sizeof(unsigned) * (max_spec_subiterations + 1),
-                                            source.stream));
-        };
-
-        {
-            for (;;) {
-                clear_flags();
-                GridImpl swap_a = source_grid.make_similar();
-                GridImpl swap_b = source_grid.make_similar();
-                swap_a.get_storage().allocate_device();
-                GridImpl *pass_source = &source_grid, *pass_target = &swap_a;
-                std::size_t iteration = params.iteration_offset;
-                std::size_t remaining = params.n_iterations;
-                bool first = true;
-                auto advance = [&](LaunchPlan const &plan, Speculation const &spec) {
-                    const unsigned n_gens =
-                        unsigned(std::min<std::size_t>(remaining, plan.fused_iterations));
-                    pass_target->get_storage().allocate_device();
-                    launch(plan, pass_source->get_storage(), pass_target->get_storage(), iteration,
-                           n_gens, &spec);
-                    iteration += n_gens;
-                    remaining -= n_gens;
-                    if (first) {
-                        pass_source = &swap_a;
-                        pass_target = &swap_b;
-                        first = false;
-                    } else {
-                        std::swap(pass_source, pass_target);
-                    }
-                };
-
-                if (!spec_probed) {
-                    // observe with the unspeculated plan, then read what changed
-                    const LaunchPlan plan0 = make_plan<F>(source.device, grid_h, grid_w,
-                                                          params.n_iterations,
-                                                          params.fused_iterations, params.tile_rows);
-                    Speculation observe{};
-                    observe.probe = true;
-                    observe.flags = spec_flags;
-                    advance(plan0, observe);
-                    last_plan = plan0;
-                    read_flags();
-                    for (unsigned q = 0; q < n_sub; q++)
-                        spec_keep[q] = ~host_flags[q] & all_planes;
-                    spec_probed = true;
-                    drop_unprofitable_speculation();
-                    clear_flags();
-                }
-
-                Speculation spec{};
-                for (unsigned q = 0; q < n_sub; q++)
-                    spec.keep[q] = spec_keep[q];
-                spec.flags = spec_flags;
-                if (remaining > 0) {
-                    const LaunchPlan plan = make_plan<F>(
-                        source.device, grid_h, grid_w, params.n_iterations, params.fused_iterations,
-                        params.tile_rows, spec.single_planes(n_sub, all_planes));
-                    last_plan = plan;
-                    while (remaining > 0)
-                        advance(plan, spec);
-                }
-                read_flags();
-                const unsigned violated = host_flags[max_spec_subiterations];
-                if (violated == 0) {
-                    pass_source->get_storage().device_written();
-                    return *pass_source;
-                }
-                // A plane believed to pass through did change: never speculate on it again and
-                // recompute this call from the untouched source grid.
-                for (unsigned q = 0; q < n_sub; q++)
-                    spec_keep[q] &= ~violated;
-                drop_unprofitable_speculation();
-                n_spec_redos++;
-                n_launches = launches_before;
-                profile_events.resize(events_before);
-            }
-        }
-    }
-
-    /// Pass-through pays through the planes that need only ONE tile buffer (taller tiles) and the
-    /// stores it saves; the kernels that support it carry per-plane buffer bookkeeping, which costs
-    /// registers. Measured (profiles/r01_s3_sweep_speculation.log): HotSpot +11 %, FDTD +19 % with
-    /// half of the cell passing through, mantle convection -11 % with one field of eleven. Below a
-    /// quarter of the cell's bytes the unspeculated kernels are used.
-    void drop_unprofitable_speculation() {
-        unsigned single = all_planes;
-        for (unsigned q = 0; q < n_sub; q++)
-            single &= spec_keep[q];
-        std::size_t bytes = 0;
-        for (std::size_t i = 0; i < Layout::n_planes; i++)
-            if ((single >> i) & 1u)
-                bytes += Layout::plane_bytes(i);
-        // ... and cells beyond 64 bytes run at the register limit of their 512-thread CTAs: the
-        // per-plane buffer bookkeeping spills there (convection: 9.2 -> 8.2 GCell-updates/s even
-        // with four of eleven fields constant in the benchmark input)
-        if (4 * bytes < sizeof(Cell) || sizeof(Cell) > 64) {
-            for (unsigned q = 0; q < n_sub; q++)
-                spec_keep[q] = 0;
-        }
-    }
-
-    bool speculation_has_nothing_left() const {
-        if (!spec_probed)
-            return false;
-        for (unsigned q = 0; q < n_sub; q++)
-            if (spec_keep[q] != 0)
-                return false;
-        return true;
-    }
+    using PassThrough = internal::PassThrough<F>;
 
     GridImpl run_simulation(GridImpl &source_grid) {
         if (params.n_iterations == 0) {
@@ -484,72 +215,138 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
                 shards.reset();
             }
         }
-        if constexpr (declared_constant != 0 && internal::speculation_capable<F>()) {
-            // fields declared constant by the cell type: no run-time detection on top of that
-            if (declared_passthrough_pays() && source_grid.get_grid_height() > 0 &&
-                source_grid.get_grid_width() > 0)
-                return run_declared(source_grid);
-        } else if constexpr (internal::speculation_capable<F>()) {
-            if (speculation_enabled() && !speculation_has_nothing_left() &&
-                source_grid.get_grid_height() > 0 && source_grid.get_grid_width() > 0)
-                return run_speculative(source_grid);
-        }
-
         auto &source = source_grid.get_storage();
-        const unsigned grid_h = unsigned(source.height);
-        const unsigned grid_w = unsigned(source.width);
+        if (source.height == 0 || source.width == 0)
+            return source_grid.make_similar();
 
-        GridImpl swap_grid_a = source_grid.make_similar();
-        if (grid_h == 0 || grid_w == 0)
-            return swap_grid_a;
-
-        const bool trace = std::getenv("STST_TRACE") != nullptr;
-        auto t_begin = std::chrono::high_resolution_clock::now();
-        auto lap = [&](const char *what) {
-            if (!trace)
-                return;
-            auto now = std::chrono::high_resolution_clock::now();
-            std::fprintf(stderr, "[stst] %-22s %9.3f ms\n", what,
-                         std::chrono::duration<double, std::milli>(now - t_begin).count());
-            t_begin = now;
-        };
-
+        lap_start = std::chrono::high_resolution_clock::now();
         source.require_device();
         lap("require_device");
 
-        const internal::LaunchPlan plan = internal::make_plan<F>(
-            source.device, grid_h, grid_w, params.n_iterations, params.fused_iterations,
-            params.tile_rows);
+        if (PassThrough::declared()) {
+            // Fields declared constant by the cell type: no observing launch and no read-back, the
+            // call stays asynchronous. With STST_VERIFY_CONSTANT_FIELDS=1 the kernels' own check of
+            // the kept planes is read after the last launch (one stream synchronisation) and a
+            // violated declaration throws std::logic_error.
+            const auto spec = pass_through.verifying(source.device, source.stream);
+            GridImpl result = run_passes(source_grid, plan_for(source, pass_through.single_planes()),
+                                         &*spec, params.iteration_offset, params.n_iterations);
+            static const bool verify = internal::env_long("STST_VERIFY_CONSTANT_FIELDS", 0) != 0;
+            if (verify) {
+                const unsigned violated = pass_through.take_violations(source.stream);
+                if (violated != 0)
+                    throw std::logic_error(
+                        "StencilStream-B200: the transition function changed a field that its cell "
+                        "type lists in Cell::constant_fields (plane mask " +
+                        std::to_string(violated) + ")");
+            }
+            return result;
+        }
+        if (PassThrough::detected() && !pass_through.nothing_left())
+            return run_detected(source_grid);
+        return run_passes(source_grid, plan_for(source, 0), nullptr, params.iteration_offset,
+                          params.n_iterations);
+    }
+
+    /**
+     * The generation loop with pass-through of DETECTED planes.
+     *
+     * The first launch this updater ever submits also *observes*: per sub-iteration, which planes
+     * came out of the transition function different from the centre cell that went in. Planes that
+     * never changed are from then on left in place by the tile sweeps instead of being copied from
+     * tile buffer to tile buffer, and planes untouched in every sub-iteration need only one tile
+     * buffer, so the tiles grow. Every launch still compares what the function returned for those
+     * planes with what went in (for a genuinely passed-through field the compiler folds that away)
+     * and reports any difference through a device flag, which is read when all launches of the call
+     * have been submitted. If a launch reports a difference — the field does change after all, e.g.
+     * FDTD's `hz_sum` once `iteration >= detect_iteration` — that plane is struck from the masks and
+     * the WHOLE call is repeated from the (never modified) source grid. The result is therefore
+     * always what the plain loop computes; the price is that such calls end with a stream
+     * synchronisation even when `blocking` is false.
+     */
+    GridImpl run_detected(GridImpl &source_grid) {
+        auto &source = source_grid.get_storage();
+        // launches and profiling events of an attempt that is discarded must not be counted
+        const std::size_t launches_before = n_launches;
+        const std::size_t events_before = profile_events.size();
+        for (;;) {
+            GridImpl result = source_grid;
+            std::size_t observed = 0; // iterations computed by the observing launch
+            if (!pass_through.probed()) {
+                const internal::Speculation observe =
+                    pass_through.observing(source.device, source.stream);
+                const internal::LaunchPlan plan = plan_for(source, 0);
+                observed = std::min<std::size_t>(params.n_iterations, plan.fused_iterations);
+                result = run_passes(source_grid, plan, &observe, params.iteration_offset, observed);
+                pass_through.read_observation(source.stream);
+            }
+            const auto spec = pass_through.verifying(source.device, source.stream);
+            if (observed < params.n_iterations)
+                result = run_passes(result, plan_for(source, pass_through.single_planes()),
+                                    spec ? &*spec : nullptr, params.iteration_offset + observed,
+                                    params.n_iterations - observed, observed > 0);
+            const unsigned violated = spec ? pass_through.take_violations(source.stream) : 0u;
+            if (violated == 0)
+                return result;
+            // A plane believed to pass through did change: never keep it again and recompute this
+            // call from the untouched source grid.
+            pass_through.drop(violated);
+            n_spec_redos++;
+            n_launches = launches_before;
+            profile_events.resize(events_before);
+        }
+    }
+
+    /**
+     * The generation loop: iterations [iteration, iteration + n_iterations) as launches of `plan`
+     * (with `spec`, if given) from `source` through two scratch grids, the second one allocated only
+     * if there is more than one launch. With `source_is_scratch` (the source is the result of an
+     * earlier launch of this call) the source grid itself serves as the second scratch grid.
+     */
+    GridImpl run_passes(GridImpl &source, internal::LaunchPlan const &plan,
+                        internal::Speculation const *spec, std::size_t iteration,
+                        std::size_t n_iterations, bool source_is_scratch = false) {
         last_plan = plan;
-        lap("make_plan");
-
         const std::size_t k = plan.fused_iterations;
-        const std::size_t n_full = params.n_iterations / k;
-        const std::size_t n_tail = params.n_iterations % k;
-        const std::size_t launches = n_full + (n_tail ? 1 : 0);
-
-        GridImpl swap_grid_b = (launches > 1) ? source_grid.make_similar() : swap_grid_a;
-        swap_grid_a.get_storage().allocate_device();
-        swap_grid_b.get_storage().allocate_device();
+        GridImpl swap_a = source.make_similar();
+        GridImpl swap_b = source_is_scratch ? source
+                          : (n_iterations > k) ? source.make_similar()
+                                               : swap_a;
+        swap_a.get_storage().allocate_device();
+        swap_b.get_storage().allocate_device();
         lap("allocate scratch grids");
 
-        GridImpl *pass_source = &source_grid;
-        GridImpl *pass_target = &swap_grid_a;
-        std::size_t iteration = params.iteration_offset;
-        for (std::size_t l = 0; l < launches; l++) {
-            const unsigned n_gens = unsigned((l < n_full) ? k : n_tail);
-            launch(plan, pass_source->get_storage(), pass_target->get_storage(), iteration, n_gens);
+        GridImpl *pass_source = &source, *pass_target = &swap_a;
+        while (n_iterations > 0) {
+            const unsigned n_gens = unsigned(std::min(n_iterations, k));
+            launch(plan, pass_source->get_storage(), pass_target->get_storage(), iteration, n_gens,
+                   spec);
             iteration += n_gens;
-            if (l == 0) {
-                pass_source = &swap_grid_a;
-                pass_target = &swap_grid_b;
-            } else {
-                std::swap(pass_source, pass_target);
-            }
+            n_iterations -= n_gens;
+            pass_source = pass_target;
+            pass_target = (pass_target == &swap_a) ? &swap_b : &swap_a;
         }
         pass_source->get_storage().device_written();
         lap("submit launches");
         return *pass_source;
+    }
+
+    internal::LaunchPlan plan_for(internal::GridStorage<Cell> const &source, unsigned single_planes) {
+        const internal::LaunchPlan plan = internal::make_plan<F>(
+            source.device, unsigned(source.height), unsigned(source.width), params.n_iterations,
+            params.fused_iterations, params.tile_rows, single_planes);
+        lap("make_plan");
+        return plan;
+    }
+
+    /// STST_TRACE: host time since the previous step of this call, on stderr.
+    void lap(const char *what) {
+        if (!std::getenv("STST_TRACE"))
+            return;
+        const auto now = std::chrono::high_resolution_clock::now();
+        std::fprintf(stderr, "[stst] %-22s %9.3f ms\n", what,
+                     std::chrono::duration<double, std::milli>(now - lap_start).count());
+        lap_start = now;
     }
 
     // ---- one update spread over several GPUs of the box (Params::cuda_devices / STST_DEVICES) ----------
@@ -687,13 +484,9 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
                 STST_RT_CHECK(stst_set_device(me));
                 set->done.push_back(std::make_unique<Event>());
             }
-            set->speculating = speculation_enabled();
-            if (set->speculating)
-                for (auto &slab : set->slabs)
-                    set->speculating = slab->enable_speculation(true) && set->speculating;
-            if (!set->speculating)
-                for (auto &slab : set->slabs)
-                    slab->enable_speculation(false);
+            set->speculating = PassThrough::detected();
+            for (auto &slab : set->slabs)
+                slab->enable_speculation(set->speculating);
             shards = std::move(set);
             return true;
         }
@@ -820,13 +613,10 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
     internal::TensorMapCache<Cell> tensor_maps;
     std::vector<std::pair<std::shared_ptr<internal::Event>, std::shared_ptr<internal::Event>>>
         profile_events;
-    // speculative plane pass-through (run_speculative)
-    bool spec_probed = false;
-    unsigned spec_keep[internal::max_spec_subiterations] = {};
-    unsigned *spec_flags = nullptr;
-    unsigned *spec_host_flags = nullptr; ///< pinned landing zone of spec_flags, allocated once
-    int spec_device = 0;
+    internal::PassThrough<F> pass_through;
     std::size_t n_spec_redos = 0;
+    std::chrono::high_resolution_clock::time_point lap_start; ///< STST_TRACE
+
     // row slabs of the multi-GPU path (run_sharded); rebuilt when grid shape or device list change
     std::unique_ptr<ShardSet> shards;
 };

@@ -9,6 +9,7 @@
  */
 #pragma once
 #include "Helpers.hpp"
+#include "PassThrough.hpp"
 #include "Planner.hpp"
 #include "Runtime.hpp"
 #include "TileKernel.hpp"
@@ -35,10 +36,6 @@ struct LaunchRegion {
     unsigned tile_h;         ///< output tile height for this launch (0: the plan's)
     int out2_row_lo = 0;     ///< optional second row range of the same launch (a slab's other
     int out2_row_hi = 0;     ///< boundary strip); empty unless out2_row_hi > out2_row_lo
-    /// One-launch pass of a slab: the tile rows that produce the first `push_rows_top` / the last
-    /// `push_rows_bottom` rows of the range run first and are the ones that take a ticket.
-    unsigned push_rows_top = 0, push_rows_bottom = 0;
-    bool boundary_first = false;
 };
 
 /**
@@ -72,32 +69,6 @@ template <typename Cell> class TensorMapCache {
     using Key = std::tuple<void *, unsigned long long, std::size_t, std::size_t, unsigned, unsigned>;
     std::map<Key, TensorMapSet> cache;
 };
-
-/**
- * Host-side state of speculative plane pass-through for one updater (see run_tile in
- * TileKernel.hpp): per sub-iteration, the planes a launch may leave in place instead of copying
- * them from tile buffer to tile buffer, and the device words through which the kernels report what
- * they observed.
- */
-struct Speculation {
-    unsigned keep[max_spec_subiterations] = {};
-    bool probe = false;          ///< the launch only observes (keep must be all-zero)
-    unsigned *flags = nullptr;   ///< device: [0, S) changed per sub-iteration, [S] violated planes
-
-    unsigned single_planes(unsigned n_sub, unsigned all_planes) const {
-        unsigned m = all_planes;
-        for (unsigned q = 0; q < n_sub; q++)
-            m &= keep[q];
-        return m;
-    }
-};
-
-/// Cells with several planes and few sub-iterations can run the pass-through kernels.
-template <typename F> constexpr bool speculation_capable() {
-    return CellLayout<typename F::Cell>::n_planes >= 2 &&
-           CellLayout<typename F::Cell>::n_planes <= 32 &&
-           F::n_subiterations <= max_spec_subiterations;
-}
 
 template <typename F> struct SweepLauncher {
     using Cell = typename F::Cell;
@@ -169,24 +140,7 @@ template <typename F> struct SweepLauncher {
         }
         geo.iteration0 = iteration0;
         const unsigned out_rows = unsigned(region.out_row_hi - region.out_row_lo);
-        const unsigned tiles_y = (out_rows + geo.tile_h - 1) / geo.tile_h;
-        geo.tiles_first = geo.tiles_x * tiles_y;
-        geo.tiles_y = tiles_y;
-        if (region.boundary_first && !second) {
-            unsigned nb_top = region.push_rows_top ? (region.push_rows_top - 1) / geo.tile_h + 1 : 0;
-            unsigned nb_bottom = 0;
-            if (region.push_rows_bottom)
-                nb_bottom = tiles_y - (out_rows > region.push_rows_bottom
-                                           ? (out_rows - region.push_rows_bottom) / geo.tile_h
-                                           : 0);
-            if (nb_top + nb_bottom >= tiles_y) { // the two sets meet: every tile row is a boundary row
-                nb_top = tiles_y;
-                nb_bottom = 0;
-            }
-            geo.nb_top = nb_top;
-            geo.nb_bottom = nb_bottom;
-            geo.ticket_ctas = (nb_top + nb_bottom) * geo.tiles_x;
-        }
+        geo.tiles_first = geo.tiles_x * ((out_rows + geo.tile_h - 1) / geo.tile_h);
         unsigned tiles_second = 0;
         if (second) {
             geo.out2_row_lo = region.out2_row_lo;
@@ -222,8 +176,6 @@ template <typename F> struct SweepLauncher {
 
         const dim3 block(plan.block_x, plan.block_y, 1);
         const dim3 grid(geo.tiles_first + tiles_second, 1, 1);
-        if (!(region.boundary_first && !second))
-            geo.ticket_ctas = grid.x; // a boundary launch of its own: every CTA takes a ticket
         auto submit = [&](auto kernel, std::size_t &configured_smem) {
             if (smem > configured_smem) {
                 cudaError_t err = cudaFuncSetAttribute(

@@ -25,8 +25,8 @@
  *                     sweep the remaining rows (they depend on no ghost row)
  *
  * so the exchange for the next pass overlaps the interior sweep of this one, and nothing but the
- * small boundary launch ever waits for a neighbour (STST_SLAB_PASS=single selects a one-launch form,
- * see pass()). Flags are waited for with
+ * small boundary launch ever waits for a neighbour (a slab too thin for two strips, or one built
+ * without `overlap`, runs its pass as one launch, see pass()). Flags are waited for with
  * cuStreamWaitValue32 (stream-ordered, no host involvement, works across processes) and raised by the
  * boundary launch itself: every CTA fences its stores system-wide and takes an atomic ticket, the
  * holder of the last ticket stores the flags (exchange_halos(), which copies with cudaMemcpy, still
@@ -44,6 +44,7 @@
 #include "FieldOps.hpp"
 #include "Helpers.hpp"
 #include "Launch.hpp"
+#include "PassThrough.hpp"
 #include "Planner.hpp"
 #include "Runtime.hpp"
 #include "TileKernel.hpp"
@@ -138,7 +139,7 @@ template <typename F> class SlabUpdate {
         unsigned fused_iterations; ///< upper bound for k; 0 = planner's choice. Must resolve to the
                                    ///< same k on every slab of a grid (checked by the caller).
         unsigned tile_rows;
-        bool overlap; ///< boundary-first scheduling (else one launch per pass)
+        bool overlap; ///< boundary strips and interior in two launches (else one launch per pass)
     };
 
     explicit SlabUpdate(Config const &config)
@@ -170,19 +171,10 @@ template <typename F> class SlabUpdate {
             peer_base[s] = nullptr;
             peer_row_lo[s] = peer_row_hi[s] = 0;
         }
-        // Fields the cell type declares constant (Cell::constant_fields, Helpers.hpp): the
-        // pass-through kernels with a compile-time keep mask; none of the backup / verify / repeat
-        // protocol of the run-time detection below is needed for them.
-        if constexpr (constant_fields_mask<Cell>() != 0 && speculation_capable<F>() &&
-                      sizeof(Cell) <= 64) {
-            if (env_long("STST_SPECULATE", 1) != 0) {
-                for (unsigned q = 0; q < n_sub; q++)
-                    spec_keep[q] = constant_fields_mask<Cell>() & all_planes;
-                spec_probed = true;
-                settle_speculation();
-                declared_active = current_spec().single_planes(n_sub, all_planes) != 0;
-            }
-        }
+        // Fields the cell type declares constant (Cell::constant_fields) pass through from the
+        // start; none of the backup / verify / repeat protocol below is needed for them.
+        if (PassThrough<F>::declared())
+            plan_passthrough();
     }
 
     SlabUpdate(SlabUpdate const &) = delete;
@@ -191,7 +183,7 @@ template <typename F> class SlabUpdate {
     ~SlabUpdate() {
         (void)stst_stream_synchronize(interior_stream);
         (void)stst_stream_synchronize(boundary_stream);
-        device_free(cfg.device, spec_flags, interior_stream);
+        pass_through.free_flags();
         device_free(cfg.device, backup_block, interior_stream);
         (void)stst_stream_synchronize(interior_stream);
         (void)stst_stream_destroy(interior_stream);
@@ -201,7 +193,7 @@ template <typename F> class SlabUpdate {
 
     // ---- speculative plane pass-through on slabs ---------------------------------------------------
     //
-    // Same mechanism as StencilUpdate::run_speculative (see there and run_tile in TileKernel.hpp): the
+    // Same mechanism as the single-GPU updater (PassThrough.hpp, run_tile in TileKernel.hpp): the
     // first pass observes which planes the transition function leaves unchanged, later passes leave
     // those planes in place, every pass verifies them. What differs is the repeat after a wrong
     // guess: a slab has no untouched source grid, and its neighbours have already consumed the rows it
@@ -210,26 +202,16 @@ template <typename F> class SlabUpdate {
     // drop_passthrough(mask), restore() and run() again (sharding.py does this with one all-reduce
     // per call). Off unless enable_speculation(true).
 
-    /// Turn pass-through on or off for the following run() calls (no-op for functors without a
-    /// second plane). Returns whether it is on.
+    /// Turn detection on or off for the following run() calls (no-op for functors that cannot pass
+    /// planes through or declare their constant fields). Returns whether it is on.
     bool enable_speculation(bool on) {
-        if (declared_active)
-            return false; // the constant fields are declared: nothing to detect, nothing to verify
-        // (cells beyond 64 bytes never profit, see settle_speculation: do not even start the
-        // protocol for them — its backup would be a third copy of a very large slab)
-        if constexpr (speculation_capable<F>() && sizeof(Cell) <= 64)
-            spec_enabled = on && env_long("STST_SPECULATE", 1) != 0;
-        return spec_enabled;
+        detecting = on && PassThrough<F>::detected();
+        return detecting;
     }
-    bool speculation_active() const { return spec_enabled && !spec_exhausted(); }
 
     /// Planes that currently pass through every sub-iteration.
     unsigned passthrough_planes() const {
-        if (declared_active)
-            return current_spec().single_planes(n_sub, all_planes);
-        if (!spec_enabled || !spec_probed)
-            return 0;
-        return current_spec().single_planes(n_sub, all_planes);
+        return (detecting || PassThrough<F>::declared()) ? pass_through.single_planes() : 0u;
     }
 
     /// Save the current generation (owned and ghost rows) so that restore() can return to it.
@@ -264,30 +246,16 @@ template <typename F> class SlabUpdate {
 
     /// Planes for which some pass since the last call saw a kept plane change. Waits for the slab.
     unsigned take_violations() {
-        if (!spec_flags)
-            return 0;
         join_streams();
-        unsigned *host = static_cast<unsigned *>(pinned_alloc(flag_bytes));
-        unsigned violated = 0;
-        try {
-            STST_RT_CHECK(stst_memcpy_d2h_async(host, spec_flags, flag_bytes, interior_stream));
-            STST_RT_CHECK(stst_stream_synchronize(interior_stream));
-            violated = host[max_spec_subiterations];
-            STST_RT_CHECK(stst_memset_async(spec_flags, 0, flag_bytes, interior_stream));
-        } catch (...) {
-            pinned_free(host);
-            throw;
-        }
-        pinned_free(host);
+        const unsigned violated = pass_through.take_violations(interior_stream);
         fork_streams();
         return violated;
     }
 
     /// Never let `planes` pass through again.
     void drop_passthrough(unsigned planes) {
-        for (unsigned q = 0; q < n_sub; q++)
-            spec_keep[q] &= ~planes;
-        settle_speculation();
+        pass_through.drop(planes);
+        plan_passthrough();
     }
 
     // ---- topology ---------------------------------------------------------------------------------
@@ -302,10 +270,7 @@ template <typename F> class SlabUpdate {
     bool has_down() const { return cfg.row_hi < cfg.grid_rows; }
     LaunchPlan const &get_plan() const { return plan; }
     /// The plan the next pass will use (taller tiles once planes pass through).
-    LaunchPlan const &get_active_plan() const {
-        return (declared_active || (spec_enabled && spec_probed && !spec_exhausted())) ? spec_plan
-                                                                                        : plan;
-    }
+    LaunchPlan const &get_active_plan() const { return passthrough_planes() ? spec_plan : plan; }
     Config const &get_config() const { return cfg; }
     std::size_t get_n_launches() const { return n_launches; }
     std::size_t get_epoch() const { return epoch; }
@@ -549,20 +514,19 @@ template <typename F> class SlabUpdate {
         std::size_t remaining = n_iterations;
         while (remaining > 0) {
             const unsigned n_gens = unsigned(std::min(remaining, k));
-            if (spec_enabled && !spec_probed) {
+            if (detecting && !pass_through.probed()) {
                 // the first pass ever observes; its result tells which planes may stay in place
-                ensure_spec_flags();
-                Speculation observe{};
-                observe.probe = true;
-                observe.flags = spec_flags;
+                const Speculation observe = pass_through.observing(cfg.device, interior_stream);
                 pass(tf, halo_value, iteration, n_gens, &observe);
-                read_observation();
-            } else if (speculation_active() || declared_active) {
-                ensure_spec_flags();
-                const Speculation spec = current_spec();
-                pass(tf, halo_value, iteration, n_gens, &spec);
+                join_streams();
+                pass_through.read_observation(interior_stream);
+                fork_streams();
+                plan_passthrough();
             } else {
-                pass(tf, halo_value, iteration, n_gens, nullptr);
+                const auto spec = passthrough_planes()
+                                      ? pass_through.verifying(cfg.device, interior_stream)
+                                      : std::nullopt;
+                pass(tf, halo_value, iteration, n_gens, spec ? &*spec : nullptr);
             }
             iteration += n_gens;
             remaining -= n_gens;
@@ -628,75 +592,12 @@ template <typename F> class SlabUpdate {
 
     void fork_streams() { join_streams(); }
 
-    static constexpr unsigned n_sub = unsigned(F::n_subiterations);
-    static constexpr unsigned all_planes =
-        Layout::n_planes >= 32 ? ~0u : ((1u << Layout::n_planes) - 1u);
-    static constexpr std::size_t flag_bytes = sizeof(unsigned) * (max_spec_subiterations + 1);
-
-    Speculation current_spec() const {
-        Speculation spec{};
-        for (unsigned q = 0; q < n_sub && q < max_spec_subiterations; q++)
-            spec.keep[q] = spec_keep[q];
-        spec.flags = spec_flags;
-        return spec;
-    }
-
-    bool spec_exhausted() const {
-        if (!spec_probed)
-            return false;
-        for (unsigned q = 0; q < n_sub && q < max_spec_subiterations; q++)
-            if (spec_keep[q] != 0)
-                return false;
-        return true;
-    }
-
-    void ensure_spec_flags() {
-        if (spec_flags)
-            return;
-        spec_flags = static_cast<unsigned *>(device_alloc(cfg.device, flag_bytes, interior_stream));
-        STST_RT_CHECK(stst_memset_async(spec_flags, 0, flag_bytes, interior_stream));
-        join_streams();
-    }
-
-    /// After the observing pass: keep what never changed, if that is worth it (same rule as
-    /// StencilUpdate::drop_unprofitable_speculation), and plan the tiles for it. The fusion depth
-    /// stays what the slab was built with — it fixes the ghost rows.
-    void read_observation() {
-        join_streams();
-        unsigned *host = static_cast<unsigned *>(pinned_alloc(flag_bytes));
-        try {
-            STST_RT_CHECK(stst_memcpy_d2h_async(host, spec_flags, flag_bytes, interior_stream));
-            STST_RT_CHECK(stst_stream_synchronize(interior_stream));
-            for (unsigned q = 0; q < n_sub && q < max_spec_subiterations; q++)
-                spec_keep[q] = ~host[q] & all_planes;
-            STST_RT_CHECK(stst_memset_async(spec_flags, 0, flag_bytes, interior_stream));
-        } catch (...) {
-            pinned_free(host);
-            throw;
-        }
-        pinned_free(host);
-        spec_probed = true;
-        settle_speculation();
-        fork_streams();
-    }
-
-    void settle_speculation() {
-        unsigned single = current_spec().single_planes(n_sub, all_planes);
-        std::size_t bytes = 0;
-        for (std::size_t i = 0; i < Layout::n_planes; i++)
-            if ((single >> i) & 1u)
-                bytes += Layout::plane_bytes(i);
-        // ... and cells beyond 64 bytes run at the register limit of their 512-thread CTAs: the
-        // per-plane buffer bookkeeping spills there (convection: 9.2 -> 8.2 GCell-updates/s even
-        // with four of eleven fields constant in the benchmark input)
-        if (4 * bytes < sizeof(Cell) || sizeof(Cell) > 64) {
-            for (unsigned q = 0; q < max_spec_subiterations; q++)
-                spec_keep[q] = 0;
-            single = 0;
-        }
+    /// Plan the tiles for the planes that pass through. The fusion depth stays what the slab was
+    /// built with: it fixes the ghost rows.
+    void plan_passthrough() {
         spec_plan = make_plan<F>(cfg.device, unsigned(cfg.row_hi - cfg.row_lo),
                                  unsigned(cfg.grid_cols), max_fused_iterations,
-                                 plan.fused_iterations, cfg.tile_rows, single);
+                                 plan.fused_iterations, cfg.tile_rows, pass_through.single_planes());
         if (spec_plan.fused_iterations != plan.fused_iterations)
             throw std::logic_error("StencilStream-B200: pass-through changed the fusion depth");
     }
@@ -780,21 +681,15 @@ template <typename F> class SlabUpdate {
             n_launches++;
         };
 
-        // How a pass is launched (cfg.overlap; STST_SLAB_PASS=split|single overrides):
-        //   split (default) — both boundary strips in ONE launch on the high-priority stream (it waits
-        //     for the neighbours' flags, pushes, and its last CTA raises their flags), the interior in
-        //     another launch that needs no flag at all: two launches per pass;
-        //   single — ONE launch over the whole slab whose tile rows are ordered boundary first, the
-        //     flags raised by the last boundary CTA. No strip tiles (which stage `strip + 2 halo` rows
-        //     for `strip` rows of output) and one launch fewer — but the WHOLE pass then waits for the
-        //     neighbours' flags, so any skew between the slabs stalls interior work that the split
-        //     form lets run: measured slower on 8 GPUs (FDTD 4608^2 565 vs 596, HotSpot 16384^2 5618
-        //     vs 5766 GCell-updates/s, profiles/r02_pass_ab_8gpu_*.json). Kept selectable;
-        //   no overlap (cfg.overlap false) — one launch in natural order, flags at its very end.
-        static const int pass_mode = [] {
-            const char *env = std::getenv("STST_SLAB_PASS");
-            return (env && std::string(env) == "single") ? 0 : 1;
-        }();
+        // How a pass is launched:
+        //   overlap — both boundary strips in ONE launch on the high-priority stream (it waits for the
+        //     neighbours' flags, pushes, and its last CTA raises their flags), the interior in another
+        //     launch that needs no flag at all: two launches per pass. (A one-launch form whose tile
+        //     rows ran boundary first was measured slower on 8 GPUs: the whole pass then waits for the
+        //     neighbours' flags, FDTD 4608^2 565 vs 596, HotSpot 16384^2 5618 vs 5766
+        //     GCell-updates/s, profiles/r02_pass_ab_8gpu_*.json.)
+        //   no overlap, or a slab too thin for two strips — one launch in natural order, every CTA
+        //     takes a ticket, the flags are raised at its very end.
         // Strips are `ghost` rows tall. Tile-high strips (no strip tile staging `ghost + 2 halo` rows
         // for `ghost` rows of output) were measured too: a boundary CTA spends ~18 us in its
         // system-scope fence and ticket whatever it computed (ncu, eight 576-row FDTD slabs: 84 strip
@@ -802,7 +697,7 @@ template <typename F> class SlabUpdate {
         // 13.09 tile rows either way, so the taller strips only moved work into the launch that
         // holds its SMs longest (N = 2: 197 vs 195 GCell-updates/s; not adopted).
         const bool can_split = cfg.overlap && neighbours && owned_rows() > 2 * ghost;
-        if (can_split && (pass_mode == 1 || nccl_comm)) {
+        if (can_split) {
             // Two launches per pass: both boundary strips (with the halo push and the flags), then
             // the interior. (The NCCL transport needs the strips finished before it can send them.)
             const std::size_t top_hi = has_up() ? cfg.row_lo + ghost : cfg.row_lo;
@@ -812,13 +707,7 @@ template <typename F> class SlabUpdate {
                 nccl_exchange(cur ^ 1); // strips out, ghost rows of the next generation in
             sweep(top_hi, bottom_lo, 0, 0, false, false, interior_stream);
         } else {
-            if (cfg.overlap && pushes) {
-                region.boundary_first = true;
-                region.push_rows_top = has_up() ? unsigned(ghost) : 0u;
-                region.push_rows_bottom = has_down() ? unsigned(ghost) : 0u;
-            }
             sweep(cfg.row_lo, cfg.row_hi, 0, 0, true, false, boundary_stream);
-            region.boundary_first = false;
             if (nccl_comm)
                 nccl_exchange(cur ^ 1);
         }
@@ -923,15 +812,13 @@ template <typename F> class SlabUpdate {
     std::size_t peer_row_lo[2], peer_row_hi[2];
     TensorMapCache<Cell> tensor_maps;
     std::unique_ptr<Event> boundary_done, interior_done;
-    // speculative plane pass-through
-    bool spec_enabled = false, spec_probed = false;
-    bool declared_active = false; ///< keep masks come from Cell::constant_fields
+    // plane pass-through; `detecting`: run-time detection on (enable_speculation)
+    PassThrough<F> pass_through;
+    bool detecting = false;
+    LaunchPlan spec_plan{};
     // NCCL halo transport (use_nccl); nullptr: peer-mapped memory and flags
     stst_nccl_comm_t nccl_comm = nullptr;
     int nccl_rank[2] = {-1, -1};
-    unsigned spec_keep[max_spec_subiterations] = {};
-    unsigned *spec_flags = nullptr;
-    LaunchPlan spec_plan{};
     void *backup_block = nullptr;
 };
 

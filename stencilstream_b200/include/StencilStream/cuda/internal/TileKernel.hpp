@@ -123,12 +123,6 @@ struct SweepGeometry {
     int out2_row_lo;         ///< a second row range produced by the same launch (both boundary strips of
     int out2_row_hi;         ///< a slab in one launch); empty unless out2_row_hi > out2_row_lo
     unsigned tiles_first;    ///< number of CTAs that work on the first range (the rest: the second)
-    // Boundary-first order of the tile rows of the first range (a slab's whole pass in ONE launch):
-    // the `nb_top` topmost and `nb_bottom` lowest tile rows — those that produce the rows the
-    // neighbouring slabs need, and the only ones that read this slab's ghost rows — get the lowest
-    // block indices, i.e. run first; both zero: natural order.
-    unsigned tiles_y, nb_top, nb_bottom;
-    unsigned ticket_ctas;    ///< the first `ticket_ctas` CTAs of the launch take a completion ticket
     unsigned tile_h, tile_w; ///< output tile extent
     unsigned halo;           ///< d = n_gens * n_subiterations * radius
     unsigned hpad;           ///< column halo, d rounded up to a multiple of CW
@@ -993,12 +987,7 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
         out_hi = geo.out2_row_hi;
     }
     const unsigned tx = tile_index % geo.tiles_x;
-    unsigned ty = tile_index / geo.tiles_x;
-    if ((geo.nb_top | geo.nb_bottom) != 0 && blockIdx.x < geo.tiles_first) {
-        const unsigned nb = geo.nb_top + geo.nb_bottom;
-        if (ty >= geo.nb_top)
-            ty = ty < nb ? geo.tiles_y - geo.nb_bottom + (ty - geo.nb_top) : geo.nb_top + (ty - nb);
-    }
+    const unsigned ty = tile_index / geo.tiles_x;
     const int tile_gy = out_lo + int(ty * geo.tile_h);
     const int tile_gx = int(tx * geo.tile_w);
     const int gy0 = tile_gy - int(geo.halo);
@@ -1020,18 +1009,20 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
             tf, halo_value, tdvs, src, dst, push, maps, geo, smem, &mbar, gy0, gx0, out_lo, out_hi);
     }
 
-    if (geo.push && push.ticket != nullptr && blockIdx.x < geo.ticket_ctas) {
+    // (`blockIdx.x < gridDim.x` always holds; without that test ptxas gives FDTD's plain kernel two
+    // registers more, see profiles/r02_kernel_resources.txt)
+    if (geo.push && push.ticket != nullptr && blockIdx.x < gridDim.x) {
         // Every thread makes its stores (own planes and the neighbours' ghost rows) visible
-        // system-wide, then the CTA takes a ticket; the holder of the last ticket knows that all
-        // ticket-taking CTAs — the whole boundary launch, or the boundary tile rows at the front of a
-        // one-launch pass — have passed their fence (fence / relaxed atomic / fence: release and
-        // acquire patterns of the PTX memory model) and raises the neighbours' flags. Those CTAs are
-        // also the only readers of this slab's ghost rows, which the neighbours overwrite next.
+        // system-wide, then the CTA takes a ticket; the holder of the last ticket knows that every
+        // CTA of the launch has passed its fence (fence / relaxed atomic / fence: release and
+        // acquire patterns of the PTX memory model) and raises the neighbours' flags. The launch that
+        // pushes is also the only reader of this slab's ghost rows, which the neighbours overwrite
+        // next.
         __threadfence_system();
         __syncthreads();
         if (threadIdx.x == 0 && threadIdx.y == 0) {
             const unsigned ticket = atomicAdd(push.ticket, 1u);
-            if (ticket == geo.ticket_ctas - 1u) {
+            if (ticket == gridDim.x - 1u) {
                 __threadfence_system();
                 if (push.flag_up != nullptr)
                     *reinterpret_cast<volatile unsigned *>(push.flag_up) = push.flag_value;

@@ -163,7 +163,7 @@ def test_tma_and_cp_async_staging_agree(monkeypatch):
     assert outs[0].tobytes() == outs[1].tobytes()
 
 
-# ---- speculative plane pass-through (StencilUpdate::run_speculative, run_tile in TileKernel.hpp) ----
+# ---- speculative plane pass-through (StencilUpdate::run_detected, run_tile in TileKernel.hpp) ----
 
 def test_passthrough_planes_are_detected():
     """HotSpot never changes `power`, FDTD never changes its four material coefficients: after the
@@ -216,6 +216,6 @@ def test_speculation_can_be_switched_off(monkeypatch, oracle_best):
     want = oracle_best.run("convection_pt", params, halo, cells, 0, 5)
     got, update = run_gpu("convection_pt", params, halo, cells, 0, 5, strict=True)
     assert got.tobytes() == want.tobytes()
-    # T is the only field this kernel never writes: 8 of 88 bytes is below the profitability
-    # threshold, so the updater falls back to the unspeculated kernels
+    # 88-byte cells have no pass-through kernels (and T, the only field this kernel never writes,
+    # would be 8 of 88 bytes, below the profitability threshold): the plain kernels run
     assert update.get_stats().passthrough_planes == 0

@@ -6,7 +6,11 @@
 For every `fused_sweep_kernel` instantiation whose mangled name contains `--match`: instruction count,
 the mnemonic histogram grouped by pipe (FP32 / FP64 / integer / shared-memory / global-memory / TMA +
 barrier / control), and the Blackwell evidence lines (UTMALDG = cp.async.bulk.tensor loads, SYNCS =
-mbarrier, STG.E.128 = 128-bit stores, LDGSTS = cp.async). Used for the profiles/r02_sass_*.txt files.
+mbarrier, STG.E.128 = 128-bit stores, LDGSTS = cp.async). Used for the profiles/r0*_sass_*.txt files.
+
+With --loops, also the body of every loop (a backward branch and what lies between its target and it)
+that holds at least 20 FFMA: what one iteration of a sweep's row loop issues, which the kernel totals
+hide when a kernel carries several loop variants.
 """
 import argparse
 import collections
@@ -46,10 +50,35 @@ def kernels(lib: Path):
         yield name, body
 
 
+def loops(lib: Path, match: str):
+    """(kernel, [(first address, instruction count, Counter of base mnemonics)]) per sweep kernel."""
+    text = subprocess.run(["cuobjdump", "-sass", str(lib)], capture_output=True, text=True).stdout
+    for part in re.split(r"\n\s*Function : ", text)[1:]:
+        name = part.split("\n", 1)[0].strip()
+        if "fused_sweep_kernel" not in name or match not in name:
+            continue
+        ins = []
+        for line in part.splitlines():
+            m = re.match(r"\s*/\*([0-9a-f]{4,})\*/\s+(?:@!?U?P\w+\s+)?([A-Z][A-Z0-9_.]*)(.*);", line)
+            if m:
+                ins.append((int(m.group(1), 16), m.group(2), m.group(3)))
+        index = {a: i for i, (a, _, _) in enumerate(ins)}
+        found = []
+        for i, (a, op, rest) in enumerate(ins):
+            t = re.search(r"0x([0-9a-f]+)", rest) if op.startswith("BRA") else None
+            if t and int(t.group(1), 16) < a and int(t.group(1), 16) in index:
+                body = ins[index[int(t.group(1), 16)]:i + 1]
+                ops = collections.Counter(o.split(".")[0] for _, o, _ in body)
+                if ops["FFMA"] >= 20:
+                    found.append((body[0][0], len(body), ops))
+        yield name, found
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--lib", type=Path, default=ROOT / "stencilstream_b200" / "libstst_workloads.so")
     ap.add_argument("--match", default="")
+    ap.add_argument("--loops", action="store_true", help="also the instruction counts of the row loops")
     args = ap.parse_args()
     for name, body in kernels(args.lib):
         if "fused_sweep_kernel" not in name or args.match not in name:
@@ -78,6 +107,13 @@ def main():
                                      "UBLKCP", "MEMBAR", "ATOM", "FFMA2"))}
         print("  evidence: " + ", ".join(f"{k} x{v}" for k, v in sorted(evidence.items())))
         print()
+    if args.loops:
+        for name, found in loops(args.lib, args.match):
+            demangled = subprocess.run(["c++filt", name], capture_output=True, text=True).stdout.strip()
+            print(f"loops of: {demangled[:150]}")
+            for start, n, ops in found:
+                counts = " ".join(f"{k} {ops[k]}" for k in ("FFMA", "FMUL", "LDS", "STS", "STG", "BAR"))
+                print(f"  loop at {start:#07x}: {n:5d} instructions, {counts}")
 
 
 if __name__ == "__main__":

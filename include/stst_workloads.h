@@ -235,6 +235,39 @@ int stst_update_apply(stst_update *update, stst_grid *source, stst_grid **result
 int stst_update_get_stats(stst_update *update, stst_update_stats *stats);
 int stst_update_destroy(stst_update *update);
 
+/* ---- grid batches (B200 extension) ---------------------------------------------------------------
+ *
+ * `members` independent grids of rows x cols cells of one workload on one device, advanced together:
+ * stst_update_apply_batch applies the update to every member with one fused launch per pass, and
+ * each member's result equals the stst_update_apply result of that member alone, bit for bit (cells
+ * outside a member read as halo_value; members never see each other). Cells cross as dense arrays of
+ * n_members x rows x cols cells, member-major. A batch runs on its own device: an update whose
+ * cuda_devices lists more than one device fails with STST_ERR_INVALID_ARGUMENT for a batch, and
+ * STST_DEVICES is ignored. At most 65535 members. */
+
+typedef struct stst_batch stst_batch;
+
+/* New, uninitialised batch. device < 0: default. */
+int stst_batch_create(const char *workload, size_t members, size_t rows, size_t cols, int device,
+                      stst_batch **batch);
+int stst_batch_destroy(stst_batch *batch);
+int stst_batch_shape(const stst_batch *batch, size_t *members, size_t *rows, size_t *cols);
+/* Members [first_member, first_member + n_members): bytes must equal n_members*rows*cols*cell_bytes
+ * and the range must lie inside the batch, else STST_ERR_RANGE. */
+int stst_batch_copy_from_host(stst_batch *batch, size_t first_member, size_t n_members,
+                              const void *cells, size_t bytes);
+int stst_batch_copy_to_host(stst_batch *batch, size_t first_member, size_t n_members, void *cells,
+                            size_t bytes);
+/* stst_grid_max_abs of member `member` (extents member-local); a member out of range: STST_ERR_RANGE. */
+int stst_batch_max_abs(stst_batch *batch, size_t member, const stst_field_extent *extents, size_t n,
+                       double *out);
+/* ONE field of every member: bytes must equal members*rows*cols*sizeof(field), else STST_ERR_RANGE. */
+int stst_batch_copy_field_to_host(stst_batch *batch, size_t field, void *values, size_t bytes);
+/* operator()(GridBatch&): *result is a new batch handle owned by the caller; `source` is not
+ * modified. Statistics as for a grid: n_processed_cells grows by n_iterations*members*rows*cols,
+ * n_launches by one per fused pass whatever the member count. */
+int stst_update_apply_batch(stst_update *update, stst_batch *source, stst_batch **result);
+
 /* ---- row slabs: the multi-GPU partitioner --------------------------------------------------------
  *
  * No counterpart in the reference (its cuda backend drives one device,

@@ -5,7 +5,8 @@ the reference's `stencil::cuda::{Grid, StencilUpdate}`) plus two C-ABI shared li
 package is the host-side mirror of that interface over the C ABI (`api`), the recipes for the
 reference's example experiments (`workloads`), and the build script (`_build`).
 """
-from .api import Grid, Params, RangeError, StencilStreamError, StencilUpdate, workload_info, workload_names
+from .api import (Grid, GridBatch, Params, RangeError, StencilStreamError, StencilUpdate, workload_info,
+                  workload_names)
 
-__all__ = ["Grid", "Params", "RangeError", "StencilStreamError", "StencilUpdate", "workload_info",
+__all__ = ["Grid", "GridBatch", "Params", "RangeError", "StencilStreamError", "StencilUpdate", "workload_info",
            "workload_names"]

@@ -197,6 +197,9 @@ WORKLOADS_SYMBOLS = [
     "stst_slab_copy_to_host", "stst_slab_copy_rows_from_host", "stst_slab_copy_rows_to_host",
     "stst_slab_exchange_halos", "stst_slab_update", "stst_slab_synchronize",
     "stst_slab_record_event",
+    "stst_batch_create", "stst_batch_destroy", "stst_batch_shape", "stst_batch_copy_from_host",
+    "stst_batch_copy_to_host", "stst_batch_max_abs", "stst_batch_copy_field_to_host",
+    "stst_update_apply_batch",
 ]
 
 _libs: dict = {}
@@ -263,5 +266,16 @@ def workloads_lib(strict: bool | None = None):
         lib.stst_update_apply.argtypes = [vp, vp, C.POINTER(vp)]
         lib.stst_update_get_stats.argtypes = [vp, C.POINTER(UpdateStats)]
         lib.stst_update_destroy.argtypes = [vp]
+        lib.stst_batch_create.argtypes = [C.c_char_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int,
+                                          C.POINTER(vp)]
+        lib.stst_batch_destroy.argtypes = [vp]
+        lib.stst_batch_shape.argtypes = [vp, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t),
+                                         C.POINTER(C.c_size_t)]
+        lib.stst_batch_copy_from_host.argtypes = [vp, C.c_size_t, C.c_size_t, vp, C.c_size_t]
+        lib.stst_batch_copy_to_host.argtypes = [vp, C.c_size_t, C.c_size_t, vp, C.c_size_t]
+        lib.stst_batch_max_abs.argtypes = [vp, C.c_size_t, C.POINTER(FieldExtent), C.c_size_t,
+                                           C.POINTER(C.c_double)]
+        lib.stst_batch_copy_field_to_host.argtypes = [vp, C.c_size_t, vp, C.c_size_t]
+        lib.stst_update_apply_batch.argtypes = [vp, vp, C.POINTER(vp)]
         _libs[key] = lib
     return _libs[key]

@@ -211,6 +211,96 @@ class Grid:
         _check(self._lib, self._lib.stst_grid_sync_to_device(self._handle))
 
 
+class GridBatch:
+    """`members` independent grids of rows x cols cells of one workload on one device (mirror of
+    `stencil::cuda::GridBatch<Cell>`), advanced together by `StencilUpdate`: one fused launch per pass
+    for all members, each member's result equal to its own grid update. Buffers are (members, rows,
+    cols) arrays of the workload's cell dtype."""
+
+    def __init__(self, workload: str, members=None, rows=None, cols=None, *, buffer=None,
+                 device: int = -1, strict: bool | None = None, _handle=None):
+        self.workload = workload
+        self._lib = _native.workloads_lib(strict)
+        self._strict = strict
+        self.dtype = CELL_DTYPES[workload]
+        if _handle is not None:
+            self._handle = _handle
+            return
+        if buffer is not None:
+            buffer = np.asarray(buffer)
+            if buffer.ndim != 3:
+                raise RangeError("a grid batch buffer must be three-dimensional (members, rows, cols)")
+            members, rows, cols = buffer.shape
+        handle = C.c_void_p()
+        _check(self._lib, self._lib.stst_batch_create(workload.encode(), int(members), int(rows),
+                                                      int(cols), int(device), C.byref(handle)))
+        self._handle = handle
+        if buffer is not None:
+            self.copy_from_buffer(buffer)
+
+    def __del__(self):
+        handle = getattr(self, "_handle", None)
+        if handle:
+            self._lib.stst_batch_destroy(handle)
+            self._handle = None
+
+    def shape(self) -> tuple[int, int, int]:
+        """(members, rows, cols)."""
+        m, r, c = C.c_size_t(), C.c_size_t(), C.c_size_t()
+        _check(self._lib, self._lib.stst_batch_shape(self._handle, C.byref(m), C.byref(r), C.byref(c)))
+        return (m.value, r.value, c.value)
+
+    def get_members(self) -> int:
+        return self.shape()[0]
+
+    def get_grid_range(self) -> tuple[int, int]:
+        """Extent of one member."""
+        return self.shape()[1:]
+
+    def copy_from_buffer(self, buffer, first_member: int = 0) -> None:
+        """Overwrite members [first_member, first_member + len(buffer)) with `buffer`, a
+        (n_members, rows, cols) array; the whole batch by default."""
+        arr = np.ascontiguousarray(buffer, dtype=self.dtype)
+        if arr.ndim != 3 or tuple(arr.shape[1:]) != self.get_grid_range():
+            raise RangeError("The target buffer has not the same size as the grid batch members")
+        _check(self._lib, self._lib.stst_batch_copy_from_host(
+            self._handle, int(first_member), arr.shape[0], arr.ctypes.data_as(C.c_void_p), arr.nbytes))
+
+    def copy_to_buffer(self, buffer: np.ndarray, first_member: int = 0) -> None:
+        """Overwrite `buffer` (C-contiguous (n_members, rows, cols) array of the cell dtype) with
+        members [first_member, first_member + n_members)."""
+        if (not isinstance(buffer, np.ndarray) or buffer.dtype != self.dtype or buffer.ndim != 3
+                or tuple(buffer.shape[1:]) != self.get_grid_range()):
+            raise RangeError("The target buffer has not the same size as the grid batch members")
+        if not buffer.flags["C_CONTIGUOUS"] or not buffer.flags["WRITEABLE"]:
+            raise ValueError("copy_to_buffer needs a writable C-contiguous array")
+        _check(self._lib, self._lib.stst_batch_copy_to_host(
+            self._handle, int(first_member), buffer.shape[0], buffer.ctypes.data_as(C.c_void_p),
+            buffer.nbytes))
+
+    def to_numpy(self) -> np.ndarray:
+        """All members as a (members, rows, cols) array."""
+        out = np.empty(self.shape(), dtype=self.dtype)
+        self.copy_to_buffer(out)
+        return out
+
+    def max_abs(self, extents, member: int) -> list[float]:
+        """`Grid.max_abs` of member `member`: [(field, rows, cols), ...] in member coordinates."""
+        extents = list(extents)
+        out = (C.c_double * max(len(extents), 1))()
+        _check(self._lib, self._lib.stst_batch_max_abs(
+            self._handle, int(member), _native.field_extents(self.workload, extents), len(extents), out))
+        return [float(out[q]) for q in range(len(extents))]
+
+    def field_to_numpy(self, field) -> np.ndarray:
+        """ONE field of every cell of every member as a (members, rows, cols) array."""
+        out = np.empty(self.shape(), dtype=_native.field_dtype(self.workload, field))
+        _check(self._lib, self._lib.stst_batch_copy_field_to_host(
+            self._handle, _native.field_index(self.workload, field),
+            out.ctypes.data_as(C.c_void_p), out.nbytes))
+        return out
+
+
 @dataclass
 class Params:
     """Mirror of `StencilUpdate::Params` (reference StencilStream/cuda/StencilUpdate.hpp:54-105);
@@ -300,10 +390,15 @@ class StencilUpdate:
         """Live reference: modifications are used by the next call (reference :152)."""
         return self.params
 
-    def __call__(self, source_grid: Grid) -> Grid:
+    def __call__(self, source_grid):
+        """operator(): a Grid gives a Grid, a GridBatch a GridBatch (every member advanced)."""
         native = self._native_params()
         _check(self._lib, self._lib.stst_update_set_params(self._handle, C.byref(native)))
         result = C.c_void_p()
+        if isinstance(source_grid, GridBatch):
+            _check(self._lib, self._lib.stst_update_apply_batch(self._handle, source_grid._handle,
+                                                                C.byref(result)))
+            return GridBatch(source_grid.workload, strict=self._strict, _handle=result)
         _check(self._lib, self._lib.stst_update_apply(self._handle, source_grid._handle,
                                                       C.byref(result)))
         return Grid(source_grid.workload, strict=self._strict, _handle=result)

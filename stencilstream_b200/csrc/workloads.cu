@@ -67,6 +67,9 @@ struct stst_update {
 struct stst_slab {
     std::unique_ptr<SlabBase> impl;
 };
+struct stst_batch {
+    std::unique_ptr<BatchBase> impl;
+};
 
 #define STST_EXPORT extern "C" __attribute__((visibility("default")))
 
@@ -265,6 +268,91 @@ STST_EXPORT int stst_update_destroy(stst_update *update) {
     return STST_OK;
 }
 
+// ---- grid batches --------------------------------------------------------------------------------------
+
+STST_EXPORT int stst_batch_create(const char *workload, size_t members, size_t rows, size_t cols,
+                                  int device, stst_batch **batch) {
+    const WorkloadEntry *e = find(workload);
+    if (!e)
+        return report(STST_ERR_UNKNOWN_WORKLOAD, std::string("unknown workload: ") +
+                                                     (workload ? workload : "(null)"));
+    if (!batch)
+        return report(STST_ERR_INVALID_ARGUMENT, "batch is null");
+    return guarded([&] {
+        *batch = new stst_batch{
+            std::unique_ptr<BatchBase>(e->make_batch(e->name, members, rows, cols, device))};
+        return STST_OK;
+    });
+}
+
+STST_EXPORT int stst_batch_destroy(stst_batch *batch) {
+    delete batch;
+    return STST_OK;
+}
+
+STST_EXPORT int stst_batch_shape(const stst_batch *batch, size_t *members, size_t *rows,
+                                 size_t *cols) {
+    if (!batch || !members || !rows || !cols)
+        return report(STST_ERR_INVALID_ARGUMENT, "null argument");
+    *members = batch->impl->members();
+    *rows = batch->impl->rows();
+    *cols = batch->impl->cols();
+    return STST_OK;
+}
+
+STST_EXPORT int stst_batch_copy_from_host(stst_batch *batch, size_t first_member, size_t n_members,
+                                          const void *cells, size_t bytes) {
+    if (!batch || (!cells && bytes != 0))
+        return report(STST_ERR_INVALID_ARGUMENT, "null argument");
+    return guarded([&] {
+        batch->impl->copy(first_member, n_members, const_cast<void *>(cells), bytes, true);
+        return STST_OK;
+    });
+}
+
+STST_EXPORT int stst_batch_copy_to_host(stst_batch *batch, size_t first_member, size_t n_members,
+                                        void *cells, size_t bytes) {
+    if (!batch || (!cells && bytes != 0))
+        return report(STST_ERR_INVALID_ARGUMENT, "null argument");
+    return guarded([&] {
+        batch->impl->copy(first_member, n_members, cells, bytes, false);
+        return STST_OK;
+    });
+}
+
+STST_EXPORT int stst_batch_max_abs(stst_batch *batch, size_t member, const stst_field_extent *extents,
+                                   size_t n, double *out) {
+    if (!batch || (n != 0 && (!extents || !out)))
+        return report(STST_ERR_INVALID_ARGUMENT, "null argument");
+    return guarded([&] {
+        batch->impl->max_abs(member, extents, n, out);
+        return STST_OK;
+    });
+}
+
+STST_EXPORT int stst_batch_copy_field_to_host(stst_batch *batch, size_t field, void *values,
+                                              size_t bytes) {
+    if (!batch || (!values && bytes != 0))
+        return report(STST_ERR_INVALID_ARGUMENT, "null argument");
+    return guarded([&] {
+        const size_t want = batch->impl->members() * batch->impl->rows() * batch->impl->cols() *
+                            batch->impl->field_bytes(field);
+        if (bytes != want)
+            return report(STST_ERR_RANGE, "The target buffer has not the same size as the field");
+        batch->impl->copy_field_to_host(field, values);
+        return STST_OK;
+    });
+}
+
+STST_EXPORT int stst_update_apply_batch(stst_update *update, stst_batch *source,
+                                        stst_batch **result) {
+    if (!update || !source || !result)
+        return report(STST_ERR_INVALID_ARGUMENT, "null argument");
+    return guarded([&] {
+        *result = new stst_batch{std::unique_ptr<BatchBase>(update->impl->apply_batch(*source->impl))};
+        return STST_OK;
+    });
+}
 
 // ---- row slabs ---------------------------------------------------------------------------------------
 

@@ -100,11 +100,61 @@ template <typename Cell> struct GridHolder final : GridBase {
     GridBase *make_similar() override { return new GridHolder(workload, grid.make_similar()); }
 };
 
+struct BatchBase {
+    virtual ~BatchBase() = default;
+    const char *workload = nullptr;
+    virtual std::size_t members() const = 0;
+    virtual std::size_t rows() const = 0;
+    virtual std::size_t cols() const = 0;
+    virtual std::size_t cell_bytes() const = 0;
+    virtual void copy(std::size_t first_member, std::size_t n_members, void *cells, std::size_t bytes,
+                      bool to_device) = 0;
+    virtual void max_abs(std::size_t member, const stst_field_extent *extents, std::size_t n,
+                         double *out) = 0;
+    virtual std::size_t field_bytes(std::size_t field) const = 0;
+    virtual void copy_field_to_host(std::size_t field, void *host) = 0;
+};
+
+template <typename Cell> struct BatchHolder final : BatchBase {
+    sc::GridBatch<Cell> batch;
+    BatchHolder(const char *name, sc::GridBatch<Cell> b) : batch(std::move(b)) { workload = name; }
+    std::size_t members() const override { return batch.get_members(); }
+    std::size_t rows() const override { return batch.get_grid_range()[0]; }
+    std::size_t cols() const override { return batch.get_grid_range()[1]; }
+    std::size_t cell_bytes() const override { return sizeof(Cell); }
+    void copy(std::size_t first_member, std::size_t n_members, void *cells, std::size_t bytes,
+              bool to_device) override {
+        if (bytes % sizeof(Cell) != 0)
+            throw std::range_error("The target buffer has not the same size as the grid batch members");
+        if (to_device)
+            batch.copy_from_host(first_member, n_members, static_cast<const Cell *>(cells),
+                                 bytes / sizeof(Cell));
+        else
+            batch.copy_to_host(first_member, n_members, static_cast<Cell *>(cells),
+                               bytes / sizeof(Cell));
+    }
+    void max_abs(std::size_t member, const stst_field_extent *extents, std::size_t n,
+                 double *out) override {
+        std::vector<sc::FieldExtent> list(n);
+        for (std::size_t q = 0; q < n; q++)
+            list[q] = sc::FieldExtent{extents[q].field, extents[q].rows, extents[q].cols};
+        const std::vector<double> result = batch.max_abs(member, list);
+        std::copy(result.begin(), result.end(), out);
+    }
+    std::size_t field_bytes(std::size_t field) const override {
+        return sc::Grid<Cell>::plane_element_bytes(field);
+    }
+    void copy_field_to_host(std::size_t field, void *host) override {
+        batch.copy_plane_to_host(field, host);
+    }
+};
+
 struct UpdateBase {
     virtual ~UpdateBase() = default;
     const char *workload = nullptr;
     virtual void set_params(const stst_update_params &p) = 0;
     virtual GridBase *apply(GridBase &source) = 0;
+    virtual BatchBase *apply_batch(BatchBase &source) = 0;
     virtual void stats(stst_update_stats &s) = 0;
 };
 
@@ -151,6 +201,14 @@ template <typename F, typename ParamBlock> struct UpdateHolder final : UpdateBas
             throw std::invalid_argument("grid belongs to a workload with a different cell type");
         sc::Grid<Cell> result = (*update)(typed->grid);
         return new GridHolder<Cell>(source.workload, result);
+    }
+
+    BatchBase *apply_batch(BatchBase &source) override {
+        auto *typed = dynamic_cast<BatchHolder<Cell> *>(&source);
+        if (!typed)
+            throw std::invalid_argument("grid batch belongs to a workload with a different cell type");
+        sc::GridBatch<Cell> result = (*update)(typed->batch);
+        return new BatchHolder<Cell>(source.workload, result);
     }
 
     void stats(stst_update_stats &s) override {
@@ -315,6 +373,7 @@ struct WorkloadEntry {
     const char *name;
     stst_workload_info info;
     GridBase *(*make_grid)(const char *, std::size_t, std::size_t, int);
+    BatchBase *(*make_batch)(const char *, std::size_t, std::size_t, std::size_t, int);
     UpdateBase *(*make_update)(const char *, const stst_update_params &);
     SlabBase *(*make_slab)(const char *, std::size_t, std::size_t, std::size_t, std::size_t, int,
                            unsigned, unsigned, bool);
@@ -334,6 +393,10 @@ template <typename F, typename ParamBlock> WorkloadEntry make_entry(const char *
         if (device < 0)
             device = sc::internal::default_device_ordinal();
         return new GridHolder<Cell>(n, sc::Grid<Cell>(r, c, device));
+    };
+    e.make_batch = [](const char *n, std::size_t members, std::size_t r, std::size_t c,
+                      int device) -> BatchBase * {
+        return new BatchHolder<Cell>(n, sc::GridBatch<Cell>(members, r, c, device));
     };
     e.make_update = [](const char *n, const stst_update_params &p) -> UpdateBase * {
         return new UpdateHolder<F, ParamBlock>(n, p);

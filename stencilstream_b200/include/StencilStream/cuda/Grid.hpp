@@ -193,30 +193,33 @@ template <typename Cell> class GridStorage {
     /**
      * Overwrite the device planes with the dense row-major array of whole cells at `src` (any host
      * memory: pinned memory is read by DMA directly, anything else through the runtime's staged
-     * pipeline, stst_memcpy_2d_auto). Returns when `src` may be reused.
+     * pipeline, stst_memcpy_2d_auto). Returns when `src` may be reused. With `n_rows`, only plane
+     * rows [row0, row0 + n_rows) are written, from the first n_rows rows of `src`.
      */
-    void transfer_to_device(const Cell *src) {
-        if (n_cells() == 0)
+    void transfer_to_device(const Cell *src, std::size_t row0 = 0,
+                            std::size_t n_rows = ~std::size_t(0)) {
+        n_rows = std::min(n_rows, height - std::min(row0, height));
+        if (n_rows * width == 0)
             return;
         allocate_device();
         Cell *from = const_cast<Cell *>(src);
         if constexpr (!Layout::is_split) {
-            STST_RT_CHECK(stst_memcpy_2d_auto(planes.base[0], planes.pitch[0] * sizeof(Cell), from,
-                                              width * sizeof(Cell), width * sizeof(Cell), height,
+            STST_RT_CHECK(stst_memcpy_2d_auto(plane_row(0, row0), planes.pitch[0] * sizeof(Cell), from,
+                                              width * sizeof(Cell), width * sizeof(Cell), n_rows,
                                               /*h2d*/ 0, device, stream));
         } else {
-            const std::size_t chunk_rows = rows_per_chunk(src);
+            const std::size_t chunk_rows = std::min(rows_per_chunk(src), n_rows);
             void *staging[2] = {device_alloc(device, chunk_rows * width * sizeof(Cell), stream),
                                 device_alloc(device, chunk_rows * width * sizeof(Cell), stream)};
             std::size_t chunk = 0;
-            for (std::size_t row = 0; row < height; row += chunk_rows, chunk++) {
-                const std::size_t rows = std::min(chunk_rows, height - row);
+            for (std::size_t row = 0; row < n_rows; row += chunk_rows, chunk++) {
+                const std::size_t rows = std::min(chunk_rows, n_rows - row);
                 const std::size_t cells = rows * width;
                 void *stage = staging[chunk & 1];
                 STST_RT_CHECK(stst_memcpy_2d_auto(stage, width * sizeof(Cell), from + row * width,
                                                   width * sizeof(Cell), width * sizeof(Cell), rows,
                                                   /*h2d*/ 0, device, stream));
-                launch_layout_kernel</*scatter=*/true>(static_cast<Cell *>(stage), row, cells);
+                launch_layout_kernel</*scatter=*/true>(static_cast<Cell *>(stage), row0 + row, cells);
             }
             device_free(device, staging[0], stream);
             device_free(device, staging[1], stream);
@@ -226,25 +229,27 @@ template <typename Cell> class GridStorage {
     }
 
     /// Copy the device planes into the dense row-major array of whole cells at `dst` (any host
-    /// memory, see transfer_to_device). Returns when `dst` holds the cells.
-    void transfer_to_host(Cell *dst) {
-        if (n_cells() == 0)
+    /// memory, see transfer_to_device). Returns when `dst` holds the cells. With `n_rows`, only
+    /// plane rows [row0, row0 + n_rows) are copied.
+    void transfer_to_host(Cell *dst, std::size_t row0 = 0, std::size_t n_rows = ~std::size_t(0)) {
+        n_rows = std::min(n_rows, height - std::min(row0, height));
+        if (n_rows * width == 0)
             return;
         allocate_device();
         if constexpr (!Layout::is_split) {
-            STST_RT_CHECK(stst_memcpy_2d_auto(planes.base[0], planes.pitch[0] * sizeof(Cell), dst,
-                                              width * sizeof(Cell), width * sizeof(Cell), height,
+            STST_RT_CHECK(stst_memcpy_2d_auto(plane_row(0, row0), planes.pitch[0] * sizeof(Cell), dst,
+                                              width * sizeof(Cell), width * sizeof(Cell), n_rows,
                                               /*d2h*/ 1, device, stream));
         } else {
-            const std::size_t chunk_rows = rows_per_chunk(dst);
+            const std::size_t chunk_rows = std::min(rows_per_chunk(dst), n_rows);
             void *staging[2] = {device_alloc(device, chunk_rows * width * sizeof(Cell), stream),
                                 device_alloc(device, chunk_rows * width * sizeof(Cell), stream)};
             std::size_t chunk = 0;
-            for (std::size_t row = 0; row < height; row += chunk_rows, chunk++) {
-                const std::size_t rows = std::min(chunk_rows, height - row);
+            for (std::size_t row = 0; row < n_rows; row += chunk_rows, chunk++) {
+                const std::size_t rows = std::min(chunk_rows, n_rows - row);
                 const std::size_t cells = rows * width;
                 void *stage = staging[chunk & 1];
-                launch_layout_kernel</*scatter=*/false>(static_cast<Cell *>(stage), row, cells);
+                launch_layout_kernel</*scatter=*/false>(static_cast<Cell *>(stage), row0 + row, cells);
                 STST_RT_CHECK(stst_memcpy_2d_auto(stage, width * sizeof(Cell), dst + row * width,
                                                   width * sizeof(Cell), width * sizeof(Cell), rows,
                                                   /*d2h*/ 1, device, stream));
@@ -253,6 +258,12 @@ template <typename Cell> class GridStorage {
             device_free(device, staging[1], stream);
         }
         STST_RT_CHECK(stst_stream_synchronize(stream));
+    }
+
+    /// Address of plane row `row` of plane `i`.
+    void *plane_row(std::size_t i, std::size_t row) const {
+        return static_cast<unsigned char *>(planes.base[i]) +
+               row * planes.pitch[i] * Layout::plane_bytes(i);
     }
 
     /// True if the host mirror exists and is the authoritative copy (or as current as the planes).

@@ -19,6 +19,12 @@
  *   - `params` is re-read on every call (:223), calls are asynchronous unless `blocking` (:133-135),
  *   - `n_processed_cells += n_iterations * H * W`, walltime accumulates (:137-141).
  *
+ * B200 extension: `operator()(GridBatch<Cell> &)` advances every member of a grid batch
+ * (cuda/GridBatch.hpp) with the same parameters, one launch per fused pass for all members; the
+ * result equals one grid update per member, bit for bit. It shares the generation loop, the planner
+ * and plane pass-through with the grid overload. A batch runs on its own device: `cuda_devices`
+ * with more than one entry throws std::invalid_argument, and STST_DEVICES does not apply.
+ *
  * What is different: instead of one launch per sweep, ceil(n_iterations / k) launches of the fused,
  * shared-memory-tiled kernel in cuda/internal/TileKernel.hpp, planned by cuda/internal/Planner.hpp.
  * Fields that a transition function only passes through are no longer copied between the tile
@@ -34,6 +40,7 @@
 #include "../Concepts.hpp"
 #include "../Stencil.hpp"
 #include "Grid.hpp"
+#include "GridBatch.hpp"
 #include "internal/Helpers.hpp"
 #include "internal/Launch.hpp"
 #include "internal/PassThrough.hpp"
@@ -71,6 +78,9 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
   public:
     /// The grid type this updater consumes and produces.
     using GridImpl = Grid<Cell>;
+
+    /// B200 extension: the grid batch type this updater also consumes and produces.
+    using GridBatchImpl = GridBatch<Cell>;
 
     struct Params {
         /// The transition function instance; may carry runtime parameters.
@@ -151,6 +161,34 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
         return result_grid;
     }
 
+    /**
+     * B200 extension: compute `n_iterations` iterations of every member of `source` and return the
+     * result as a new batch (the source itself for `n_iterations == 0`); the source is not modified.
+     * Semantics as for a grid, per member; `n_processed_cells` grows by n_iterations * members *
+     * H * W, `get_n_launches()` by one per fused pass.
+     */
+    GridBatchImpl operator()(GridBatchImpl &source) {
+        if (params.cuda_devices.size() > 1)
+            throw std::invalid_argument("StencilStream-B200: a grid batch runs on one device; "
+                                        "Params::cuda_devices lists several");
+        if (source.get_members() > internal::max_batch_members)
+            throw std::invalid_argument("StencilStream-B200: a grid batch holds at most " +
+                                        std::to_string(internal::max_batch_members) + " members");
+        auto walltime_start = std::chrono::high_resolution_clock::now();
+
+        GridBatchImpl result = run_simulation(source);
+
+        if (params.blocking) {
+            STST_RT_CHECK(stst_stream_synchronize(source.get_storage().stream));
+        }
+
+        auto walltime_end = std::chrono::high_resolution_clock::now();
+        walltime += std::chrono::duration<double>(walltime_end - walltime_start).count();
+        n_processed_cells +=
+            params.n_iterations * source.get_storage().height * source.get_storage().width;
+        return result;
+    }
+
     /// Live reference to the parameters; changes apply to the next call of `operator()`.
     Params &get_params() { return params; }
 
@@ -195,7 +233,13 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
   private:
     using PassThrough = internal::PassThrough<F>;
 
-    GridImpl run_simulation(GridImpl &source_grid) {
+    /// Members of a grid batch, 0 for a grid (the launches' LaunchRegion::members).
+    static unsigned members_of(GridImpl &) { return 0; }
+    static unsigned members_of(GridBatchImpl &batch) { return unsigned(batch.get_members()); }
+
+    // G: GridImpl or GridBatchImpl
+    template <typename G> G run_simulation(G &source_grid) {
+        constexpr bool is_batch = std::is_same_v<G, GridBatchImpl>;
         if (params.n_iterations == 0) {
             return source_grid;
         }
@@ -205,7 +249,7 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
                 " but the source grid lives on device " +
                 std::to_string(source_grid.get_storage().device) +
                 "; updates run where their grid is (create the grid on that device)");
-        {
+        if constexpr (!is_batch) {
             const std::vector<int> devices = resolve_devices();
             if (devices.size() > 1 && source_grid.get_grid_height() > 0 &&
                 source_grid.get_grid_width() > 0) {
@@ -229,8 +273,10 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
             // the kept planes is read after the last launch (one stream synchronisation) and a
             // violated declaration throws std::logic_error.
             const auto spec = pass_through.verifying(source.device, source.stream);
-            GridImpl result = run_passes(source_grid, plan_for(source, pass_through.single_planes()),
-                                         &*spec, params.iteration_offset, params.n_iterations);
+            const unsigned members = members_of(source_grid);
+            G result = run_passes(source_grid,
+                                  plan_for(source, pass_through.single_planes(), members), &*spec,
+                                  params.iteration_offset, params.n_iterations);
             static const bool verify = internal::env_long("STST_VERIFY_CONSTANT_FIELDS", 0) != 0;
             if (verify) {
                 const unsigned violated = pass_through.take_violations(source.stream);
@@ -244,8 +290,8 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
         }
         if (PassThrough::detected() && !pass_through.nothing_left())
             return run_detected(source_grid);
-        return run_passes(source_grid, plan_for(source, 0), nullptr, params.iteration_offset,
-                          params.n_iterations);
+        return run_passes(source_grid, plan_for(source, 0, members_of(source_grid)), nullptr,
+                          params.iteration_offset, params.n_iterations);
     }
 
     /**
@@ -264,25 +310,26 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
      * always what the plain loop computes; the price is that such calls end with a stream
      * synchronisation even when `blocking` is false.
      */
-    GridImpl run_detected(GridImpl &source_grid) {
+    template <typename G> G run_detected(G &source_grid) {
         auto &source = source_grid.get_storage();
+        const unsigned members = members_of(source_grid);
         // launches and profiling events of an attempt that is discarded must not be counted
         const std::size_t launches_before = n_launches;
         const std::size_t events_before = profile_events.size();
         for (;;) {
-            GridImpl result = source_grid;
+            G result = source_grid;
             std::size_t observed = 0; // iterations computed by the observing launch
             if (!pass_through.probed()) {
                 const internal::Speculation observe =
                     pass_through.observing(source.device, source.stream);
-                const internal::LaunchPlan plan = plan_for(source, 0);
+                const internal::LaunchPlan plan = plan_for(source, 0, members);
                 observed = std::min<std::size_t>(params.n_iterations, plan.fused_iterations);
                 result = run_passes(source_grid, plan, &observe, params.iteration_offset, observed);
                 pass_through.read_observation(source.stream);
             }
             const auto spec = pass_through.verifying(source.device, source.stream);
             if (observed < params.n_iterations)
-                result = run_passes(result, plan_for(source, pass_through.single_planes()),
+                result = run_passes(result, plan_for(source, pass_through.single_planes(), members),
                                     spec ? &*spec : nullptr, params.iteration_offset + observed,
                                     params.n_iterations - observed, observed > 0);
             const unsigned violated = spec ? pass_through.take_violations(source.stream) : 0u;
@@ -303,24 +350,25 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
      * if there is more than one launch. With `source_is_scratch` (the source is the result of an
      * earlier launch of this call) the source grid itself serves as the second scratch grid.
      */
-    GridImpl run_passes(GridImpl &source, internal::LaunchPlan const &plan,
-                        internal::Speculation const *spec, std::size_t iteration,
-                        std::size_t n_iterations, bool source_is_scratch = false) {
+    template <typename G>
+    G run_passes(G &source, internal::LaunchPlan const &plan, internal::Speculation const *spec,
+                 std::size_t iteration, std::size_t n_iterations, bool source_is_scratch = false) {
         last_plan = plan;
         const std::size_t k = plan.fused_iterations;
-        GridImpl swap_a = source.make_similar();
-        GridImpl swap_b = source_is_scratch ? source
-                          : (n_iterations > k) ? source.make_similar()
-                                               : swap_a;
+        const unsigned members = members_of(source);
+        G swap_a = source.make_similar();
+        G swap_b = source_is_scratch ? source
+                   : (n_iterations > k) ? source.make_similar()
+                                        : swap_a;
         swap_a.get_storage().allocate_device();
         swap_b.get_storage().allocate_device();
         lap("allocate scratch grids");
 
-        GridImpl *pass_source = &source, *pass_target = &swap_a;
+        G *pass_source = &source, *pass_target = &swap_a;
         while (n_iterations > 0) {
             const unsigned n_gens = unsigned(std::min(n_iterations, k));
             launch(plan, pass_source->get_storage(), pass_target->get_storage(), iteration, n_gens,
-                   spec);
+                   spec, members);
             iteration += n_gens;
             n_iterations -= n_gens;
             pass_source = pass_target;
@@ -331,10 +379,13 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
         return *pass_source;
     }
 
-    internal::LaunchPlan plan_for(internal::GridStorage<Cell> const &source, unsigned single_planes) {
+    /// Plan for the grid `source`, or for the batch of `members` members it holds.
+    internal::LaunchPlan plan_for(internal::GridStorage<Cell> const &source, unsigned single_planes,
+                                  unsigned members) {
         const internal::LaunchPlan plan = internal::make_plan<F>(
-            source.device, unsigned(source.height), unsigned(source.width), params.n_iterations,
-            params.fused_iterations, params.tile_rows, single_planes);
+            source.device, unsigned(members ? source.height / members : source.height),
+            unsigned(source.width), params.n_iterations, params.fused_iterations, params.tile_rows,
+            single_planes, std::max(members, 1u));
         lap("make_plan");
         return plan;
     }
@@ -572,19 +623,22 @@ template <concepts::TransitionFunction F, bool split_cell_structure = false> cla
         return result;
     }
 
+    /// One fused launch over the grid in `src`, or over every member of the batch it holds.
     void launch(internal::LaunchPlan const &plan, internal::GridStorage<Cell> &src,
                 internal::GridStorage<Cell> &dst, std::size_t iteration0, unsigned n_gens,
-                internal::Speculation const *spec = nullptr) {
+                internal::Speculation const *spec, unsigned members) {
         using namespace internal;
+        const std::size_t grid_h = members ? src.height / members : src.height;
         LaunchRegion region{};
         region.device = src.device;
-        region.grid_h = unsigned(src.height);
+        region.grid_h = unsigned(grid_h);
         region.grid_w = unsigned(src.width);
         region.buf_row0 = 0;
         region.buf_rows = src.height;
         region.out_row_lo = 0;
-        region.out_row_hi = int(src.height);
+        region.out_row_hi = int(grid_h);
         region.tile_h = 0;
+        region.members = members;
 
         std::shared_ptr<Event> start, stop;
         if (params.profiling) {

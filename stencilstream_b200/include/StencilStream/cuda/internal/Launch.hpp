@@ -20,6 +20,7 @@
 #include <stdexcept>
 #include <string>
 #include <tuple>
+#include <type_traits>
 
 namespace stencil {
 namespace cuda {
@@ -36,7 +37,13 @@ struct LaunchRegion {
     unsigned tile_h;         ///< output tile height for this launch (0: the plan's)
     int out2_row_lo = 0;     ///< optional second row range of the same launch (a slab's other
     int out2_row_hi = 0;     ///< boundary strip); empty unless out2_row_hi > out2_row_lo
+    /// > 0: the planes hold a grid batch of this many members of grid_h x grid_w cells each, stacked
+    /// by rows (fused_sweep_batch_kernel); every row range above is then member-local.
+    unsigned members = 0;
 };
+
+/// Members one batch launch can hold (gridDim.y).
+inline constexpr unsigned max_batch_members = 65535;
 
 /**
  * TMA descriptors, encoded once per (plane set, box) and reused: cuTensorMapEncodeTiled costs a
@@ -101,6 +108,9 @@ template <typename F> struct SweepLauncher {
             throw std::invalid_argument("StencilStream-B200: illegal number of fused iterations");
         if (region.out_row_hi <= region.out_row_lo || region.grid_w == 0)
             return;
+        const bool batch = region.members > 0;
+        if (region.members > max_batch_members || (batch && (push || region.buf_row0 != 0)))
+            throw std::invalid_argument("StencilStream-B200: illegal grid batch launch");
 
         SweepGeometry geo{};
         geo.grid_h = region.grid_h;
@@ -175,8 +185,8 @@ template <typename F> struct SweepLauncher {
         }
 
         const dim3 block(plan.block_x, plan.block_y, 1);
-        const dim3 grid(geo.tiles_first + tiles_second, 1, 1);
-        auto submit = [&](auto kernel, std::size_t &configured_smem) {
+        const dim3 grid(geo.tiles_first + tiles_second, batch ? region.members : 1u, 1);
+        auto submit = [&](auto kernel, std::size_t &configured_smem, auto batch_c) {
             if (smem > configured_smem) {
                 cudaError_t err = cudaFuncSetAttribute(
                     kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
@@ -186,24 +196,33 @@ template <typename F> struct SweepLauncher {
                                              cudaGetErrorString(err));
                 configured_smem = smem;
             }
-            kernel<<<grid, block, smem, static_cast<cudaStream_t>(stream)>>>(
-                tf, halo_value, tdvs, src, dst, push ? *push : no_push, *maps, geo);
+            if constexpr (decltype(batch_c)::value)
+                kernel<<<grid, block, smem, static_cast<cudaStream_t>(stream)>>>(
+                    tf, halo_value, tdvs, src, dst, *maps, geo);
+            else
+                kernel<<<grid, block, smem, static_cast<cudaStream_t>(stream)>>>(
+                    tf, halo_value, tdvs, src, dst, push ? *push : no_push, *maps, geo);
         };
-        static std::size_t configured_smem_per_device[2][64] = {};
+        // [spec][batch][device]
+        static std::size_t configured_smem_per_device[2][2][64] = {};
+        auto submit_kind = [&](auto spec_c) {
+            constexpr bool kSpec = decltype(spec_c)::value;
+            if (batch)
+                submit(fused_sweep_batch_kernel<F, CW, kMode, fixed_block_x<Cell>(),
+                                                max_threads_per_cta<Cell>(), 1, kSpec>,
+                       configured_smem_per_device[kSpec][1][region.device & 63], std::true_type{});
+            else
+                submit(fused_sweep_kernel<F, CW, kMode, fixed_block_x<Cell>(),
+                                          max_threads_per_cta<Cell>(), 1, kSpec>,
+                       configured_smem_per_device[kSpec][0][region.device & 63], std::false_type{});
+        };
         if constexpr (speculation_capable<F>()) {
-            if (spec) {
-                submit(fused_sweep_kernel<F, CW, kMode, fixed_block_x<Cell>(),
-                                          max_threads_per_cta<Cell>(), 1, true>,
-                       configured_smem_per_device[1][region.device & 63]);
-            } else {
-                submit(fused_sweep_kernel<F, CW, kMode, fixed_block_x<Cell>(),
-                                          max_threads_per_cta<Cell>(), 1, false>,
-                       configured_smem_per_device[0][region.device & 63]);
-            }
+            if (spec)
+                submit_kind(std::true_type{});
+            else
+                submit_kind(std::false_type{});
         } else {
-            submit(fused_sweep_kernel<F, CW, kMode, fixed_block_x<Cell>(),
-                                      max_threads_per_cta<Cell>(), 1, false>,
-                   configured_smem_per_device[0][region.device & 63]);
+            submit_kind(std::false_type{});
         }
         cudaError_t err = cudaGetLastError();
         if (err != cudaSuccess)

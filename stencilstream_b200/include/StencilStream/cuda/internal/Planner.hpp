@@ -202,6 +202,31 @@ TileShape shape_for(unsigned k, unsigned n_sub, unsigned radius, unsigned cw, un
 }
 
 /**
+ * Small grids: with fewer CTAs than the GPU holds at once, a launch lasts as long as ONE CTA's
+ * load -> sweeps -> store sequence, however few SMs take part. Shorter tiles spread the grid over
+ * just under one resident set of CTAs (a second, mostly empty wave costs more than it gains:
+ * 1024^2 HotSpot, 29-row tiles 166, 13-row tiles 205, 19-row tiles — 270 CTAs on 296 slots —
+ * 249 GCell-updates/s; Jacobi 340 -> 408; 2048^2 and larger are unaffected;
+ * profiles/r01_s3_sweep_small_grids.log). Not below twice the halo (tile efficiency).
+ *
+ * Returns the tile height for `members` grids of grid_h x grid_w cells launched together (a grid
+ * batch): the CTAs of all members count against the `slots` resident CTAs, so a batch of many small
+ * members keeps the tall tiles `tile_h` of the unshrunk plan. A result below `tile_h` asks for the
+ * shorter tile. Host-only.
+ */
+inline unsigned small_grid_tile_rows(unsigned tile_h, unsigned halo, unsigned tile_w,
+                                     unsigned grid_h, unsigned grid_w, unsigned members,
+                                     unsigned slots) {
+    const unsigned long long tiles_x = (std::max(grid_w, 1u) + tile_w - 1) / tile_w;
+    const unsigned long long tile_columns = tiles_x * std::max(members, 1u);
+    const unsigned want_tile_rows =
+        unsigned(std::max<unsigned long long>(1ull, slots * 95ull / 100ull / tile_columns));
+    const unsigned shrunk =
+        std::max(2 * halo, (std::max(grid_h, 1u) + want_tile_rows - 1) / want_tile_rows);
+    return std::min(tile_h, shrunk);
+}
+
+/**
  * Plan launches for transition function `F` on `device`.
  *
  * The heuristic models the time per cell-iteration of a k-fused launch as
@@ -213,7 +238,7 @@ TileShape shape_for(unsigned k, unsigned n_sub, unsigned radius, unsigned cw, un
 template <typename F>
 LaunchPlan make_plan(int device, unsigned grid_h, unsigned grid_w, std::size_t n_iterations,
                      unsigned fused_override, unsigned tile_rows_override,
-                     unsigned single_planes = 0) {
+                     unsigned single_planes = 0, unsigned members = 1) {
     using Cell = typename F::Cell;
     using L = CellLayout<Cell>;
     constexpr unsigned cw = unsigned(column_group_width<Cell>());
@@ -339,18 +364,11 @@ LaunchPlan make_plan(int device, unsigned grid_h, unsigned grid_w, std::size_t n
                 "StencilStream-B200: cell type too large for a shared-memory tile");
     }
 
-    // Small grids: with fewer CTAs than the GPU holds at once, a launch lasts as long as ONE CTA's
-    // load -> sweeps -> store sequence, however few SMs take part. Shorter tiles spread the grid over
-    // just under one resident set of CTAs (a second, mostly empty wave costs more than it gains:
-    // 1024^2 HotSpot, 29-row tiles 166, 13-row tiles 205, 19-row tiles — 270 CTAs on 296 slots —
-    // 249 GCell-updates/s; Jacobi 340 -> 408; 2048^2 and larger are unaffected;
-    // profiles/r01_s3_sweep_small_grids.log). Not below twice the halo (tile efficiency).
+    // Small grids (small_grid_tile_rows): shorter tiles, unless the batch fills the GPU anyway.
     if (tile_rows_override == 0 && best.tile_h > 2 * best.halo) {
-        const unsigned tiles_x = (std::max(grid_w, 1u) + best.tile_w - 1) / best.tile_w;
         const unsigned slots = unsigned(std::max(info.sm_count, 1)) * ctas_per_sm;
-        const unsigned want_tile_rows = std::max(1u, slots * 95u / 100u / tiles_x);
-        const unsigned tile_h =
-            std::max(2 * best.halo, (std::max(grid_h, 1u) + want_tile_rows - 1) / want_tile_rows);
+        const unsigned tile_h = small_grid_tile_rows(best.tile_h, best.halo, best.tile_w, grid_h,
+                                                     grid_w, members, slots);
         if (tile_h < best.tile_h) {
             const TileShape shrunk =
                 shape_for<Cell>(best_k, n_sub, radius, cw, col_align, block_x, tile_h,

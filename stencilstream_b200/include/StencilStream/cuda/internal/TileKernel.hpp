@@ -1010,7 +1010,9 @@ sweep_pair(F const &tf, typename F::TimeDependentValue const &tdv1,
 // one tile: stage, run all fused sweeps, write back
 // ------------------------------------------------------------------------------------------------
 
-template <typename F, int CW, bool kInterior, int kMode, int kTX, bool kSpec>
+// kBatch: instantiated separately for fused_sweep_batch_kernel (same code), so that the batch kernel
+// leaves the code generated for fused_sweep_kernel exactly as it is
+template <typename F, int CW, bool kInterior, int kMode, int kTX, bool kSpec, bool kBatch = false>
 __device__ __forceinline__ void
 run_tile(F const &tf, typename F::Cell const &halo_value,
          TdvArray<typename F::TimeDependentValue> const &tdvs, PlaneSet const &src,
@@ -1282,6 +1284,64 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
                 __threadfence_system();
             }
         }
+    }
+}
+
+/**
+ * The fused kernel over a grid batch: member b of the batch occupies plane rows [b * H, (b + 1) * H)
+ * of `src` and `dst`, where H = geo.grid_h is the member extent. Grid: blockIdx.y is the member,
+ * blockIdx.x = ty * tiles_x + tx the tile within it, so a launch holds at most 65535 members
+ * (gridDim.y). Everything the tile code sees is member-local (`stencil.id`, `grid_range`, the
+ * interior test, the halo patching and the re-imposition of `halo_value`); only addresses into the
+ * planes carry the member's row offset, through buf_row0. A border tile's TMA box may reach into
+ * the neighbouring members' rows: those rows lie outside [0, H) and are overwritten with
+ * `halo_value` exactly like rows outside a single grid. One row range per launch, no halo push.
+ * (A kernel of its own rather than a branch in fused_sweep_kernel, whose code stays as it is.)
+ */
+template <typename F, int CW, int kMode, int kTX, int kMaxThreads, int kMinBlocks, bool kSpec = false>
+__global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
+    fused_sweep_batch_kernel(const __grid_constant__ F tf,
+                             const __grid_constant__ typename F::Cell halo_value,
+                             const __grid_constant__ TdvArray<typename F::TimeDependentValue> tdvs,
+                             const __grid_constant__ PlaneSet src,
+                             const __grid_constant__ PlaneSet dst,
+                             const __grid_constant__ TensorMapSet maps,
+                             const __grid_constant__ SweepGeometry geo) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ unsigned long long mbar;
+
+    if (geo.use_tma) {
+        if (threadIdx.x == 0 && threadIdx.y == 0) {
+            mbarrier_init(&mbar, 1);
+            fence_mbarrier_init();
+        }
+        __syncthreads();
+    }
+
+    SweepGeometry member = geo;
+    member.buf_row0 = geo.buf_row0 - int(blockIdx.y * geo.grid_h);
+    member.push = 0u;
+    const HaloPush no_push{};
+
+    // as in fused_sweep_kernel, member-local
+    const int out_lo = geo.out_row_lo, out_hi = geo.out_row_hi;
+    const unsigned tx = blockIdx.x % geo.tiles_x;
+    const unsigned ty = blockIdx.x / geo.tiles_x;
+    const int tile_gy = out_lo + int(ty * geo.tile_h);
+    const int tile_gx = int(tx * geo.tile_w);
+    const int gy0 = tile_gy - int(geo.halo);
+    const int gx0 = tile_gx - int(geo.hpad);
+    const bool interior = gy0 >= 0 && tile_gy + int(geo.tile_h + geo.halo) <= int(geo.grid_h) &&
+                          tile_gy + int(geo.tile_h) <= out_hi && gx0 >= 1 &&
+                          tile_gx + int(geo.tile_w + geo.hpad) + 1 <= int(geo.grid_w);
+
+    if (interior) {
+        run_tile<F, CW, true, kMode, kTX, kSpec, true>(tf, halo_value, tdvs, src, dst, no_push, maps,
+                                                       member, smem, &mbar, gy0, gx0, out_lo, out_hi);
+    } else {
+        run_tile<F, CW, false, (kMode == window_reload ? window_reload : window_shift), kTX, kSpec,
+                 true>(tf, halo_value, tdvs, src, dst, no_push, maps, member, smem, &mbar, gy0, gx0,
+                       out_lo, out_hi);
     }
 }
 

@@ -34,6 +34,14 @@ inline int report(int code, std::string message) {
     return code;
 }
 
+/// The C ABI's extents as the `FieldExtent`s of Grid::max_abs and its batch and slab counterparts.
+inline std::vector<sc::FieldExtent> field_extents(const stst_field_extent *extents, std::size_t n) {
+    std::vector<sc::FieldExtent> list(n);
+    for (std::size_t q = 0; q < n; q++)
+        list[q] = sc::FieldExtent{extents[q].field, extents[q].rows, extents[q].cols};
+    return list;
+}
+
 // ---- type-erased object model -------------------------------------------------------------------
 
 struct GridBase {
@@ -81,10 +89,7 @@ template <typename Cell> struct GridHolder final : GridBase {
     }
     bool host_pinned() override { return grid.get_storage().host_mirror_is_pinned(); }
     void max_abs(const stst_field_extent *extents, std::size_t n, double *out) override {
-        std::vector<sc::FieldExtent> list(n);
-        for (std::size_t q = 0; q < n; q++)
-            list[q] = sc::FieldExtent{extents[q].field, extents[q].rows, extents[q].cols};
-        const std::vector<double> result = grid.max_abs(list);
+        const std::vector<double> result = grid.max_abs(field_extents(extents, n));
         std::copy(result.begin(), result.end(), out);
     }
     std::size_t field_bytes(std::size_t field) const override {
@@ -135,10 +140,7 @@ template <typename Cell> struct BatchHolder final : BatchBase {
     }
     void max_abs(std::size_t member, const stst_field_extent *extents, std::size_t n,
                  double *out) override {
-        std::vector<sc::FieldExtent> list(n);
-        for (std::size_t q = 0; q < n; q++)
-            list[q] = sc::FieldExtent{extents[q].field, extents[q].rows, extents[q].cols};
-        const std::vector<double> result = batch.max_abs(member, list);
+        const std::vector<double> result = batch.max_abs(member, field_extents(extents, n));
         std::copy(result.begin(), result.end(), out);
     }
     std::size_t field_bytes(std::size_t field) const override {
@@ -323,13 +325,8 @@ template <typename F, typename ParamBlock> struct SlabHolder final : SlabBase {
     }
     void exchange() override { slab->exchange_halos(); }
     void max_abs(const stst_field_extent *extents, std::size_t n, double *out) override {
-        std::vector<std::size_t> planes(n), rows(n), cols(n);
-        for (std::size_t q = 0; q < n; q++) {
-            planes[q] = extents[q].field;
-            rows[q] = extents[q].rows;
-            cols[q] = extents[q].cols;
-        }
-        slab->max_abs(n, planes.data(), rows.data(), cols.data(), out);
+        const std::vector<double> result = slab->max_abs(field_extents(extents, n));
+        std::copy(result.begin(), result.end(), out);
     }
     std::size_t field_bytes(std::size_t field) const override {
         return sc::Grid<Cell>::plane_element_bytes(field);

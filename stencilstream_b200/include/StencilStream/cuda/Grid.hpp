@@ -8,18 +8,17 @@
  * (reference Grid.hpp:97).
  *
  * What is different underneath: the reference keeps an array-of-structs `sycl::buffer<Cell, 2>` and
- * lets the SYCL runtime migrate it. Here the device copy is a set of row-major planes, one per
- * `Cell::fields` entry (see cuda/internal/Helpers.hpp), each row padded to 128 bytes, allocated from
- * the runtime's stream-ordered pool; the host copy is a lazily created pinned array-of-structs
- * mirror that only exists once host code asks for a `GridAccessor` or a buffer copy. Transfers
- * between the two are explicit (chunked pinned copies plus a layout-conversion kernel) and happen
- * at the same points where SYCL would migrate: accessor construction and the next update.
+ * lets the SYCL runtime migrate it. Here the device copy is a plane image (cuda/internal/PlaneImage.hpp:
+ * one row-major plane per `Cell::fields` entry), allocated from the runtime's stream-ordered pool; the
+ * host copy is a lazily created pinned array-of-structs mirror that only exists once host code asks
+ * for a `GridAccessor` or a buffer copy. Transfers between the two are explicit (`transfer_cells`)
+ * and happen at the same points where SYCL would migrate: accessor construction and the next update.
  */
 #pragma once
 #include "internal/FieldOps.hpp"
 #include "internal/Helpers.hpp"
+#include "internal/PlaneImage.hpp"
 #include "internal/Runtime.hpp"
-#include "internal/TileKernel.hpp"
 
 #include <sycl/sycl.hpp>
 
@@ -35,13 +34,6 @@
 
 namespace stencil {
 namespace cuda {
-
-/// B200 extension: "field `plane` (index into `Cell::fields`; 0 for scalar cells), restricted to the
-/// first `rows` rows and `cols` columns of the grid" — the operand of `Grid::max_abs`.
-struct FieldExtent {
-    std::size_t plane;
-    std::size_t rows, cols;
-};
 
 namespace internal {
 
@@ -62,8 +54,8 @@ template <typename Cell> class GridStorage {
 
     GridStorage(std::size_t height, std::size_t width, int device)
         : height(height), width(width), device(device), stream(default_stream(device)),
-          planes{}, device_block(nullptr), host(nullptr), host_is_pinned(false),
-          host_current(true), device_current(true) {
+          image(width, height), planes{}, device_block(nullptr), host(nullptr),
+          host_is_pinned(false), host_current(true), device_current(true) {
         if (height > 0x7fffffffull || width > 0x7fffffffull)
             throw std::range_error("StencilStream-B200 grids are limited to 2^31-1 rows/columns");
     }
@@ -83,33 +75,12 @@ template <typename Cell> class GridStorage {
         }
     }
 
-    /// Elements between consecutive rows of plane `i` (row byte pitch is a multiple of 128).
-    static std::size_t plane_pitch(std::size_t i, std::size_t width) {
-        const std::size_t elem = Layout::plane_bytes(i);
-        // Smallest element count whose byte size is a multiple of both `elem` and 128.
-        std::size_t pitch = std::max<std::size_t>(width, 1);
-        while ((pitch * elem) % 128 != 0)
-            pitch++;
-        return pitch;
-    }
-
     /// Make sure the device planes exist (contents unspecified if they had to be created).
     void allocate_device() {
         if (device_block)
             return;
-        std::size_t offsets[Layout::n_planes];
-        std::size_t total = 0;
-        for (std::size_t i = 0; i < Layout::n_planes; i++) {
-            offsets[i] = total;
-            const std::size_t bytes =
-                plane_pitch(i, width) * std::max<std::size_t>(height, 1) * Layout::plane_bytes(i);
-            total += (bytes + 255) / 256 * 256;
-        }
-        device_block = device_alloc(device, total, stream);
-        for (std::size_t i = 0; i < Layout::n_planes; i++) {
-            planes.base[i] = static_cast<unsigned char *>(device_block) + offsets[i];
-            planes.pitch[i] = plane_pitch(i, width);
-        }
+        device_block = device_alloc(device, image.bytes, stream);
+        planes = image.planes(device_block);
     }
 
     void allocate_host() {
@@ -142,7 +113,7 @@ template <typename Cell> class GridStorage {
     void require_device() {
         allocate_device();
         if (!device_current) {
-            upload();
+            transfer(host, /*to_device=*/true);
             device_current = true;
         }
     }
@@ -151,7 +122,7 @@ template <typename Cell> class GridStorage {
     void require_host() {
         allocate_host();
         if (!host_current) {
-            download();
+            transfer(host, /*to_device=*/false);
             host_current = true;
         }
     }
@@ -171,99 +142,23 @@ template <typename Cell> class GridStorage {
     const std::size_t height, width;
     const int device;
     const stst_stream_t stream;
+    const PlaneImage<Cell> image;
     PlaneSet planes;
 
-  private:
-    static constexpr std::size_t staging_bytes = std::size_t(64) << 20;
-
-    std::size_t rows_per_chunk(const void *host_ptr) const {
-        // Pageable host memory goes through the runtime's pinned staging ring, which drains at the
-        // end of every call: use larger device-side chunks there so that the drain is amortised.
-        int pinned = 0;
-        (void)stst_host_is_pinned(host_ptr, &pinned);
-        const std::size_t budget = pinned ? staging_bytes : 4 * staging_bytes;
-        const std::size_t row_bytes = std::max<std::size_t>(width * sizeof(Cell), 1);
-        return std::max<std::size_t>(1, std::min<std::size_t>(height, budget / row_bytes));
-    }
-
-    void upload() { transfer_to_device(host); }
-    void download() { transfer_to_host(host); }
-
-  public:
     /**
-     * Overwrite the device planes with the dense row-major array of whole cells at `src` (any host
-     * memory: pinned memory is read by DMA directly, anything else through the runtime's staged
-     * pipeline, stst_memcpy_2d_auto). Returns when `src` may be reused. With `n_rows`, only plane
-     * rows [row0, row0 + n_rows) are written, from the first n_rows rows of `src`.
+     * Copy between the dense row-major array of whole cells at `cells` (any host memory, see
+     * transfer_cells) and the device planes: into them if `to_device`, else out of them. Returns
+     * when `cells` may be reused, or holds the cells. With `n_rows`, only plane rows
+     * [row0, row0 + n_rows) are copied, to or from the first n_rows rows of `cells`.
      */
-    void transfer_to_device(const Cell *src, std::size_t row0 = 0,
-                            std::size_t n_rows = ~std::size_t(0)) {
+    void transfer(Cell *cells, bool to_device, std::size_t row0 = 0,
+                  std::size_t n_rows = ~std::size_t(0)) {
         n_rows = std::min(n_rows, height - std::min(row0, height));
         if (n_rows * width == 0)
             return;
         allocate_device();
-        Cell *from = const_cast<Cell *>(src);
-        if constexpr (!Layout::is_split) {
-            STST_RT_CHECK(stst_memcpy_2d_auto(plane_row(0, row0), planes.pitch[0] * sizeof(Cell), from,
-                                              width * sizeof(Cell), width * sizeof(Cell), n_rows,
-                                              /*h2d*/ 0, device, stream));
-        } else {
-            const std::size_t chunk_rows = std::min(rows_per_chunk(src), n_rows);
-            void *staging[2] = {device_alloc(device, chunk_rows * width * sizeof(Cell), stream),
-                                device_alloc(device, chunk_rows * width * sizeof(Cell), stream)};
-            std::size_t chunk = 0;
-            for (std::size_t row = 0; row < n_rows; row += chunk_rows, chunk++) {
-                const std::size_t rows = std::min(chunk_rows, n_rows - row);
-                const std::size_t cells = rows * width;
-                void *stage = staging[chunk & 1];
-                STST_RT_CHECK(stst_memcpy_2d_auto(stage, width * sizeof(Cell), from + row * width,
-                                                  width * sizeof(Cell), width * sizeof(Cell), rows,
-                                                  /*h2d*/ 0, device, stream));
-                launch_layout_kernel</*scatter=*/true>(static_cast<Cell *>(stage), row0 + row, cells);
-            }
-            device_free(device, staging[0], stream);
-            device_free(device, staging[1], stream);
-        }
-        // The caller may modify the source right after this returns: finish reading it now.
+        transfer_cells<Cell>(device, stream, planes, width, row0, n_rows, cells, to_device);
         STST_RT_CHECK(stst_stream_synchronize(stream));
-    }
-
-    /// Copy the device planes into the dense row-major array of whole cells at `dst` (any host
-    /// memory, see transfer_to_device). Returns when `dst` holds the cells. With `n_rows`, only
-    /// plane rows [row0, row0 + n_rows) are copied.
-    void transfer_to_host(Cell *dst, std::size_t row0 = 0, std::size_t n_rows = ~std::size_t(0)) {
-        n_rows = std::min(n_rows, height - std::min(row0, height));
-        if (n_rows * width == 0)
-            return;
-        allocate_device();
-        if constexpr (!Layout::is_split) {
-            STST_RT_CHECK(stst_memcpy_2d_auto(plane_row(0, row0), planes.pitch[0] * sizeof(Cell), dst,
-                                              width * sizeof(Cell), width * sizeof(Cell), n_rows,
-                                              /*d2h*/ 1, device, stream));
-        } else {
-            const std::size_t chunk_rows = std::min(rows_per_chunk(dst), n_rows);
-            void *staging[2] = {device_alloc(device, chunk_rows * width * sizeof(Cell), stream),
-                                device_alloc(device, chunk_rows * width * sizeof(Cell), stream)};
-            std::size_t chunk = 0;
-            for (std::size_t row = 0; row < n_rows; row += chunk_rows, chunk++) {
-                const std::size_t rows = std::min(chunk_rows, n_rows - row);
-                const std::size_t cells = rows * width;
-                void *stage = staging[chunk & 1];
-                launch_layout_kernel</*scatter=*/false>(static_cast<Cell *>(stage), row0 + row, cells);
-                STST_RT_CHECK(stst_memcpy_2d_auto(stage, width * sizeof(Cell), dst + row * width,
-                                                  width * sizeof(Cell), width * sizeof(Cell), rows,
-                                                  /*d2h*/ 1, device, stream));
-            }
-            device_free(device, staging[0], stream);
-            device_free(device, staging[1], stream);
-        }
-        STST_RT_CHECK(stst_stream_synchronize(stream));
-    }
-
-    /// Address of plane row `row` of plane `i`.
-    void *plane_row(std::size_t i, std::size_t row) const {
-        return static_cast<unsigned char *>(planes.base[i]) +
-               row * planes.pitch[i] * Layout::plane_bytes(i);
     }
 
     /// True if the host mirror exists and is the authoritative copy (or as current as the planes).
@@ -271,35 +166,6 @@ template <typename Cell> class GridStorage {
     bool host_mirror_is_pinned() const { return host != nullptr && host_is_pinned; }
 
   private:
-    template <bool scatter>
-    void launch_layout_kernel(Cell *staging, std::size_t plane_row0, std::size_t cells) {
-#if defined(__CUDACC__)
-        int current_device = -1;
-        if (cudaGetDevice(&current_device) != cudaSuccess || current_device != device)
-            cudaSetDevice(device); // the stream belongs to this grid's device
-        const unsigned block = 256;
-        const unsigned grid =
-            unsigned(std::min<std::size_t>((cells + block - 1) / block, std::size_t(148) * 16));
-        if constexpr (scatter) {
-            scatter_cells_kernel<Cell><<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(
-                staging, planes, width, plane_row0, cells);
-        } else {
-            gather_cells_kernel<Cell><<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(
-                staging, planes, width, plane_row0, cells);
-        }
-        cudaError_t err = cudaGetLastError();
-        if (err != cudaSuccess)
-            throw std::runtime_error(std::string("StencilStream-B200: layout kernel launch failed: ") +
-                                     cudaGetErrorString(err));
-#else
-        (void)staging;
-        (void)plane_row0;
-        (void)cells;
-        throw std::runtime_error("StencilStream-B200 must be compiled with nvcc for sm_100a; "
-                                 "there is no CPU fallback");
-#endif
-    }
-
     void *device_block;
     Cell *host;
     bool host_is_pinned;
@@ -348,7 +214,7 @@ template <typename Cell> class Grid {
     /// B200 extension: `copy_from_buffer` from a dense row-major array of height x width cells. The
     /// cells go straight to the device (no intermediate host mirror).
     void copy_from_host(const Cell *cells) {
-        storage->transfer_to_device(cells);
+        storage->transfer(const_cast<Cell *>(cells), /*to_device=*/true);
         storage->device_written();
     }
 
@@ -358,7 +224,7 @@ template <typename Cell> class Grid {
             STST_RT_CHECK(stst_host_memcpy(static_cast<void *>(cells), storage->host_data(),
                                            storage->n_cells() * sizeof(Cell)));
         } else {
-            storage->transfer_to_host(cells);
+            storage->transfer(cells, /*to_device=*/false);
         }
     }
 
@@ -438,24 +304,10 @@ template <typename Cell> class Grid {
      * grid to the host). Waits for pending device work on the grid.
      */
     std::vector<double> max_abs(std::vector<FieldExtent> const &extents) {
-        std::vector<double> result(extents.size());
         storage->require_device();
-        for (std::size_t first = 0; first < extents.size();
-             first += internal::max_field_reductions) {
-            internal::FieldReduceBatch batch{};
-            batch.n = unsigned(
-                std::min<std::size_t>(extents.size() - first, internal::max_field_reductions));
-            for (unsigned q = 0; q < batch.n; q++) {
-                FieldExtent const &e = extents[first + q];
-                batch.req[q].plane = unsigned(e.plane);
-                batch.req[q].row_lo = 0;
-                batch.req[q].row_hi = unsigned(std::min(e.rows, storage->height));
-                batch.req[q].cols = unsigned(std::min(e.cols, storage->width));
-            }
-            internal::reduce_max_abs<Cell>(storage->device, storage->stream, storage->planes, batch,
-                                           result.data() + first);
-        }
-        return result;
+        return internal::reduce_max_abs<Cell>(
+            storage->device, storage->stream, storage->planes,
+            internal::field_requests(extents, storage->width, 0, storage->height, 0));
     }
 
     /// B200 extension: `max_abs` of the field `Cell::*Field` over the first `rows` x `cols` cells.

@@ -4,9 +4,9 @@
  * launch per pass whatever B is (ensembles and parameter studies of small grids, which one launch
  * per member would leave launch-bound).
  *
- * Storage: the members are stacked by rows in ONE set of planes, member b at plane rows
- * [b * H, (b + 1) * H), with the pitch and alignment of a `Grid<Cell>` of B * H x W cells; uploads,
- * downloads and the per-field operations are the grid's own, with row offsets. The update treats
+ * Storage: the members are stacked by rows in ONE plane image (cuda/internal/PlaneImage.hpp) of
+ * B * H x W cells, member b at plane rows [b * H, (b + 1) * H): the `GridStorage` of a `Grid<Cell>` of
+ * that extent. Uploads, downloads and the per-field operations are the grid's own, with row offsets. The update treats
  * every member as a grid of its own: each member's neighbours outside its H x W cells read as
  * `halo_value`, so the result equals B separate grid updates, bit for bit.
  *
@@ -55,7 +55,8 @@ template <typename Cell> class GridBatch {
                         std::size_t n_cells) {
         check_range(first_member, n_members, n_cells);
         storage->require_device();
-        storage->transfer_to_device(cells, first_member * rows, n_members * rows);
+        storage->transfer(const_cast<Cell *>(cells), /*to_device=*/true, first_member * rows,
+                          n_members * rows);
         storage->device_written();
     }
 
@@ -70,7 +71,7 @@ template <typename Cell> class GridBatch {
                       std::size_t n_cells) {
         check_range(first_member, n_members, n_cells);
         storage->require_device();
-        storage->transfer_to_host(cells, first_member * rows, n_members * rows);
+        storage->transfer(cells, /*to_device=*/false, first_member * rows, n_members * rows);
     }
 
     /// The whole batch into a dense array of members x rows x cols cells.
@@ -80,25 +81,10 @@ template <typename Cell> class GridBatch {
     std::vector<double> max_abs(std::size_t member, std::vector<FieldExtent> const &extents) {
         if (member >= members)
             throw std::range_error("StencilStream-B200: no such member in the grid batch");
-        std::vector<double> result(extents.size());
         storage->require_device();
-        const std::size_t row0 = member * rows;
-        for (std::size_t first = 0; first < extents.size();
-             first += internal::max_field_reductions) {
-            internal::FieldReduceBatch batch{};
-            batch.n = unsigned(
-                std::min<std::size_t>(extents.size() - first, internal::max_field_reductions));
-            for (unsigned q = 0; q < batch.n; q++) {
-                FieldExtent const &e = extents[first + q];
-                batch.req[q].plane = unsigned(e.plane);
-                batch.req[q].row_lo = unsigned(row0);
-                batch.req[q].row_hi = unsigned(row0 + std::min(e.rows, rows));
-                batch.req[q].cols = unsigned(std::min(e.cols, storage->width));
-            }
-            internal::reduce_max_abs<Cell>(storage->device, storage->stream, storage->planes, batch,
-                                           result.data() + first);
-        }
-        return result;
+        return internal::reduce_max_abs<Cell>(
+            storage->device, storage->stream, storage->planes,
+            internal::field_requests(extents, storage->width, 0, rows, member * rows));
     }
 
     /// ONE field of every cell of every member into the dense host array `dst` (members x rows x

@@ -1,6 +1,6 @@
 /*
- * StencilStream-B200 — per-field device operations on a grid's planes: max-norm reductions and
- * single-field transfers.
+ * StencilStream-B200 — per-field device operations on the plane image (PlaneImage.hpp) of a grid,
+ * grid batch or slab: max-norm reductions and single-field transfers.
  *
  * The reference has no counterpart: its applications obtain such values on the host, through a
  * `GridAccessor` that migrates the WHOLE array-of-structs buffer first. Mantle convection does so
@@ -10,6 +10,9 @@
  * convection.cpp:460-477). Because `cuda::Grid` stores one plane per `Cell::fields` entry, both are
  * plane-local here:
  *
+ *   field_requests          the requests of `FieldExtent`s (grid coordinates) on an image that holds
+ *                           some of the grid's rows from some plane row on: a grid all rows from 0,
+ *                           batch member m rows [0, H) from m * H, a slab its owned rows from `ghost`.
  *   reduce_max_abs_kernel   one launch evaluates up to `max_field_reductions` requests
  *                           max{ |plane[r][c]| : row_lo <= r < row_hi, c < cols } — every request
  *                           streams its sub-rectangle once with 128-bit loads; HBM-bound,
@@ -29,6 +32,7 @@
 #include <limits>
 #include <stdexcept>
 #include <type_traits>
+#include <vector>
 
 #if defined(__CUDACC__)
     #include <cuda_runtime.h>
@@ -36,6 +40,14 @@
 
 namespace stencil {
 namespace cuda {
+
+/// B200 extension: "field `plane` (index into `Cell::fields`; 0 for scalar cells), restricted to the
+/// first `rows` rows and `cols` columns of the grid" — the operand of `Grid::max_abs`.
+struct FieldExtent {
+    std::size_t plane;
+    std::size_t rows, cols;
+};
+
 namespace internal {
 
 inline constexpr unsigned max_field_reductions = 8;
@@ -164,59 +176,83 @@ __global__ void __launch_bounds__(reduce_block_threads)
 #endif // __CUDACC__
 
 /**
- * Evaluate `batch` on `planes` (device `device`, in order on `stream`) and wait for the result.
- * out[q] = max |v| of request q, -infinity if the request covers no cell.
+ * Evaluate `requests` on `planes` (device `device`, in order on `stream`), one launch per
+ * `max_field_reductions` of them, and wait for the results. result[q] = max |v| of request q,
+ * -infinity if the request covers no cell.
  */
 template <typename Cell>
-inline void reduce_max_abs(int device, stst_stream_t stream, PlaneSet const &planes,
-                           FieldReduceBatch const &batch, double *out) {
+inline std::vector<double> reduce_max_abs(int device, stst_stream_t stream, PlaneSet const &planes,
+                                          std::vector<FieldReduceRequest> const &requests) {
+    std::vector<double> result(requests.size());
 #if defined(__CUDACC__)
-    if (batch.n == 0)
-        return;
-    if (batch.n > max_field_reductions)
-        throw std::invalid_argument("StencilStream-B200: too many reductions in one batch");
-    unsigned max_rows = 0;
-    for (unsigned q = 0; q < batch.n; q++) {
-        auto const &rq = batch.req[q];
+    for (auto const &rq : requests) {
         if (rq.plane >= CellLayout<Cell>::n_planes || !plane_is_arithmetic<Cell>(rq.plane))
             throw std::invalid_argument("StencilStream-B200: field cannot be reduced (no such "
                                         "field, or not an arithmetic type)");
-        if (rq.row_hi > rq.row_lo && rq.cols > 0)
-            max_rows = std::max(max_rows, rq.row_hi - rq.row_lo);
     }
     const std::size_t bytes = sizeof(unsigned long long) * max_field_reductions;
-    unsigned long long *host_keys = static_cast<unsigned long long *>(pinned_alloc(bytes));
-    void *dev_keys = nullptr;
-    try {
-        dev_keys = device_alloc(device, bytes, stream);
-        STST_RT_CHECK(stst_memset_async(dev_keys, 0, bytes, stream));
-        if (max_rows > 0) {
-            int current_device = -1;
-            if (cudaGetDevice(&current_device) != cudaSuccess || current_device != device)
-                cudaSetDevice(device); // the stream belongs to `device`
-            const unsigned ctas = std::min<unsigned>(max_rows, 148u * 8u);
-            reduce_max_abs_kernel<Cell>
-                <<<ctas, reduce_block_threads, 0, static_cast<cudaStream_t>(stream)>>>(
-                    planes, batch, static_cast<unsigned long long *>(dev_keys));
-            if (cudaGetLastError() != cudaSuccess)
-                throw std::runtime_error("StencilStream-B200: reduction kernel launch failed");
+    for (std::size_t first = 0; first < requests.size(); first += max_field_reductions) {
+        FieldReduceBatch batch{};
+        batch.n = unsigned(std::min<std::size_t>(requests.size() - first, max_field_reductions));
+        unsigned max_rows = 0;
+        for (unsigned q = 0; q < batch.n; q++) {
+            auto const &rq = batch.req[q] = requests[first + q];
+            if (rq.row_hi > rq.row_lo && rq.cols > 0)
+                max_rows = std::max(max_rows, rq.row_hi - rq.row_lo);
         }
-        STST_RT_CHECK(stst_memcpy_d2h_async(host_keys, dev_keys, bytes, stream));
-        STST_RT_CHECK(stst_stream_synchronize(stream));
-    } catch (...) {
+        unsigned long long *host_keys = static_cast<unsigned long long *>(pinned_alloc(bytes));
+        void *dev_keys = nullptr;
+        try {
+            dev_keys = device_alloc(device, bytes, stream);
+            STST_RT_CHECK(stst_memset_async(dev_keys, 0, bytes, stream));
+            if (max_rows > 0) {
+                select_device(device);
+                const unsigned ctas = std::min<unsigned>(max_rows, 148u * 8u);
+                reduce_max_abs_kernel<Cell>
+                    <<<ctas, reduce_block_threads, 0, static_cast<cudaStream_t>(stream)>>>(
+                        planes, batch, static_cast<unsigned long long *>(dev_keys));
+                if (cudaGetLastError() != cudaSuccess)
+                    throw std::runtime_error("StencilStream-B200: reduction kernel launch failed");
+            }
+            STST_RT_CHECK(stst_memcpy_d2h_async(host_keys, dev_keys, bytes, stream));
+            STST_RT_CHECK(stst_stream_synchronize(stream));
+        } catch (...) {
+            device_free(device, dev_keys, stream);
+            pinned_free(host_keys);
+            throw;
+        }
+        for (unsigned q = 0; q < batch.n; q++)
+            result[first + q] = max_abs_from_key(host_keys[q]);
         device_free(device, dev_keys, stream);
         pinned_free(host_keys);
-        throw;
     }
-    for (unsigned q = 0; q < batch.n; q++)
-        out[q] = max_abs_from_key(host_keys[q]);
-    device_free(device, dev_keys, stream);
-    pinned_free(host_keys);
 #else
-    (void)device, (void)stream, (void)planes, (void)batch, (void)out;
-    throw std::runtime_error("StencilStream-B200 must be compiled with nvcc for sm_100a; "
-                             "there is no CPU fallback");
+    (void)device, (void)stream, (void)planes;
+    if (!requests.empty())
+        throw std::runtime_error("StencilStream-B200 must be compiled with nvcc for sm_100a; "
+                                 "there is no CPU fallback");
 #endif
+    return result;
+}
+
+/**
+ * The requests that evaluate `extents` (grid coordinates: rows [0, extent.rows), columns
+ * [0, extent.cols)) on an image whose plane rows from `plane_row0` on hold the grid rows
+ * [row_lo, row_hi) of a grid `width` columns wide. Rows and columns outside those are not covered;
+ * an extent that covers none of them gives an empty request.
+ */
+inline std::vector<FieldReduceRequest> field_requests(std::vector<FieldExtent> const &extents,
+                                                      std::size_t width, std::size_t row_lo,
+                                                      std::size_t row_hi, std::size_t plane_row0) {
+    std::vector<FieldReduceRequest> requests(extents.size());
+    for (std::size_t q = 0; q < extents.size(); q++) {
+        const std::size_t hi = std::min(extents[q].rows, row_hi);
+        requests[q].plane = unsigned(extents[q].plane);
+        requests[q].row_lo = unsigned(plane_row0);
+        requests[q].row_hi = unsigned(hi > row_lo ? plane_row0 + (hi - row_lo) : plane_row0);
+        requests[q].cols = unsigned(std::min(extents[q].cols, width));
+    }
+    return requests;
 }
 
 /**

@@ -177,12 +177,7 @@ template <typename F> struct SweepLauncher {
 
         static const HaloPush no_push{};
 
-        int current_device = -1;
-        if (cudaGetDevice(&current_device) != cudaSuccess || current_device != region.device) {
-            if (cudaSetDevice(region.device) != cudaSuccess)
-                throw std::runtime_error("StencilStream-B200: cannot select CUDA device " +
-                                         std::to_string(region.device));
-        }
+        select_device(region.device);
 
         const dim3 block(plan.block_x, plan.block_y, 1);
         const dim3 grid(geo.tiles_first + tiles_second, batch ? region.members : 1u, 1);

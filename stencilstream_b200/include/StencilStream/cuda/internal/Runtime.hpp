@@ -1,12 +1,16 @@
 /*
  * StencilStream-B200 — C++ veneer over the C-ABI device runtime (include/stst_rt.h).
  *
- * Turns status codes into exceptions and owns nothing else. The reference obtains the same services
- * from the SYCL runtime (sycl::queue / sycl::buffer / sycl::event; reference
+ * Turns status codes into exceptions and makes a device current before a kernel launch
+ * (select_device); it owns nothing else. The reference obtains the same services from the SYCL
+ * runtime (sycl::queue / sycl::buffer / sycl::event; reference
  * StencilStream/cuda/StencilUpdate.hpp:124-135 and cuda/Grid.hpp:66-134).
  */
 #pragma once
 #include <stst_rt.h>
+#if defined(__CUDACC__)
+    #include <cuda_runtime.h>
+#endif
 
 #include <cstddef>
 #include <stdexcept>
@@ -32,6 +36,21 @@ inline void check(int status, const char *call) {
 }
 
 #define STST_RT_CHECK(call) ::stencil::cuda::internal::check((call), #call)
+
+/// Make `device` current for the calling thread if it is not: a kernel launched on a stream must be
+/// launched with the stream's device current.
+inline void select_device(int device) {
+#if defined(__CUDACC__)
+    int current = -1;
+    if (cudaGetDevice(&current) != cudaSuccess || current != device) {
+        if (cudaSetDevice(device) != cudaSuccess)
+            throw std::runtime_error("StencilStream-B200: cannot select CUDA device " +
+                                     std::to_string(device));
+    }
+#else
+    (void)device; // code compiled without nvcc launches no kernel
+#endif
+}
 
 inline stst_stream_t default_stream(int device) {
     stst_stream_t s = nullptr;

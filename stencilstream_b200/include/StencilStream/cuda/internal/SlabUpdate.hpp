@@ -10,8 +10,10 @@
  *
  * Decomposition. GPU g owns the global rows [row_lo, row_hi) of every plane and keeps `ghost` further
  * rows on each side, ghost = k * n_sub * r for the fusion depth k fixed at construction. A slab holds
- * two complete plane sets (ping/pong) and two 32-bit flags in ONE cudaMalloc block, so that a single
- * IPC handle (or, within a process, a peer mapping) makes all of it addressable by the neighbours.
+ * two plane images (PlaneImage.hpp; ping/pong) and two 32-bit flags in ONE cudaMalloc block, so that
+ * a single IPC handle (or, within a process, a peer mapping) makes all of it addressable by the
+ * neighbours. Cells move to and from the host with the grid's own `transfer_cells`, asynchronously
+ * on the slab's stream for uploads.
  *
  * One pass (two launches that together advance the slab by n_gens <= k iterations), epoch e:
  *
@@ -45,6 +47,7 @@
 #include "Helpers.hpp"
 #include "Launch.hpp"
 #include "PassThrough.hpp"
+#include "PlaneImage.hpp"
 #include "Planner.hpp"
 #include "Runtime.hpp"
 #include "TileKernel.hpp"
@@ -72,46 +75,28 @@ template <int = 0> __global__ void raise_flag_kernel(volatile unsigned *flag, un
 }
 #endif
 
-/// Byte layout of a slab's single device allocation; a pure function of its shape, so that a
+/// Byte layout of a slab's single device allocation: the flag words, then two plane images
+/// (ping/pong) of owned_rows + 2 * ghost rows each. A pure function of the slab's shape, so that a
 /// neighbour can address into a mapped slab knowing only that slab's row range.
 template <typename Cell> struct SlabLayout {
-    using Layout = CellLayout<Cell>;
     /// [0]: flag_from_up, [1]: flag_from_down, [8]: ticket counter of the boundary launches
     static constexpr std::size_t flag_bytes = 256;
     static constexpr int ticket_word = 8;
 
-    std::size_t width, owned_rows, ghost, buf_rows;
-    std::size_t pitch[max_planes];        ///< elements between rows, per plane
-    std::size_t plane_offset[2][max_planes]; ///< byte offset of plane i of buffer b
+    std::size_t owned_rows, buf_rows;
+    PlaneImage<Cell> image; ///< the layout of either buffer
     std::size_t total_bytes;
 
     SlabLayout(std::size_t width, std::size_t owned_rows, std::size_t ghost)
-        : width(width), owned_rows(owned_rows), ghost(ghost), buf_rows(owned_rows + 2 * ghost),
-          pitch{}, plane_offset{}, total_bytes(0) {
-        std::size_t offset = flag_bytes;
-        for (int b = 0; b < 2; b++) {
-            for (std::size_t i = 0; i < Layout::n_planes; i++) {
-                const std::size_t elem = Layout::plane_bytes(i);
-                std::size_t p = std::max<std::size_t>(width, 1);
-                while ((p * elem) % 128 != 0)
-                    p++;
-                pitch[i] = p;
-                plane_offset[b][i] = offset;
-                const std::size_t bytes = p * buf_rows * elem;
-                offset += (bytes + 255) / 256 * 256;
-            }
-        }
-        total_bytes = offset;
+        : owned_rows(owned_rows), buf_rows(owned_rows + 2 * ghost), image(width, buf_rows),
+          total_bytes(flag_bytes + 2 * image.bytes) {}
+
+    /// Start of buffer `buffer` (0 or 1) of the slab allocated at `base`.
+    unsigned char *buffer_begin(void *base, int buffer) const {
+        return static_cast<unsigned char *>(base) + flag_bytes + buffer * image.bytes;
     }
 
-    PlaneSet planes(void *base, int buffer) const {
-        PlaneSet set{};
-        for (std::size_t i = 0; i < Layout::n_planes; i++) {
-            set.base[i] = static_cast<unsigned char *>(base) + plane_offset[buffer][i];
-            set.pitch[i] = pitch[i];
-        }
-        return set;
-    }
+    PlaneSet planes(void *base, int buffer) const { return image.planes(buffer_begin(base, buffer)); }
 
     static unsigned *flag(void *base, int which) { return static_cast<unsigned *>(base) + which; }
 };
@@ -225,11 +210,11 @@ template <typename F> class SlabUpdate {
                 STST_RT_CHECK(stst_stream_wait_value32_geq(interior_stream, my_flag(s),
                                                            unsigned(epoch + 1)));
         }
-        const std::size_t bytes = plane_set_bytes();
+        const std::size_t bytes = layout.image.bytes;
         if (!backup_block)
             backup_block = device_alloc(cfg.device, bytes, interior_stream);
-        STST_RT_CHECK(stst_memcpy_d2d_async(backup_block, plane_set_begin(int(epoch & 1)), bytes,
-                                            interior_stream));
+        STST_RT_CHECK(stst_memcpy_d2d_async(backup_block, layout.buffer_begin(base, int(epoch & 1)),
+                                            bytes, interior_stream));
         fork_streams();
     }
 
@@ -239,8 +224,8 @@ template <typename F> class SlabUpdate {
         if (!backup_block)
             throw std::logic_error("StencilStream-B200: restore() without backup()");
         join_streams();
-        STST_RT_CHECK(stst_memcpy_d2d_async(plane_set_begin(int(epoch & 1)), backup_block,
-                                            plane_set_bytes(), interior_stream));
+        STST_RT_CHECK(stst_memcpy_d2d_async(layout.buffer_begin(base, int(epoch & 1)), backup_block,
+                                            layout.image.bytes, interior_stream));
         fork_streams();
     }
 
@@ -328,7 +313,8 @@ template <typename F> class SlabUpdate {
     /// staged in host memory at once).
     void upload_rows(const Cell *cells, std::size_t first_row, std::size_t n_rows) {
         check_row_range(first_row, n_rows);
-        transfer</*to_device=*/true>(const_cast<Cell *>(cells), first_row, n_rows);
+        transfer_cells<Cell>(cfg.device, interior_stream, current_planes(), cfg.grid_cols,
+                             ghost + first_row, n_rows, const_cast<Cell *>(cells), /*to_device=*/true);
     }
 
     /// Copy the owned rows of the current generation into `cells`. Returns after the copy is done.
@@ -337,33 +323,22 @@ template <typename F> class SlabUpdate {
     void download_rows(Cell *cells, std::size_t first_row, std::size_t n_rows) {
         check_row_range(first_row, n_rows);
         join_streams();
-        transfer</*to_device=*/false>(cells, first_row, n_rows);
+        transfer_cells<Cell>(cfg.device, interior_stream, current_planes(), cfg.grid_cols,
+                             ghost + first_row, n_rows, cells, /*to_device=*/false);
         STST_RT_CHECK(stst_stream_synchronize(interior_stream));
     }
 
     /**
-     * Max-norms of single fields over this slab's share of the extents (see Grid::max_abs): request q
-     * covers the GLOBAL rows [0, rows[q]) and columns [0, cols[q]) of plane planes[q]; out[q] is the
-     * maximum over the rows this slab owns (-infinity if it owns none of them). The caller combines
-     * the slabs' values with `max` (an all-reduce across ranks). Waits for the slab's pending work.
+     * Max-norms of single fields over this slab's share of the extents (see Grid::max_abs): the
+     * extents are in GLOBAL rows; result[q] is the maximum over the rows this slab owns (-infinity if
+     * it owns none of them). The caller combines the slabs' values with `max` (an all-reduce across
+     * ranks). Waits for the slab's pending work.
      */
-    void max_abs(std::size_t n, const std::size_t *planes_idx, const std::size_t *rows,
-                 const std::size_t *cols, double *out) {
+    std::vector<double> max_abs(std::vector<FieldExtent> const &extents) {
         join_streams();
-        const PlaneSet planes = layout.planes(base, int(epoch & 1));
-        for (std::size_t first = 0; first < n; first += max_field_reductions) {
-            FieldReduceBatch batch{};
-            batch.n = unsigned(std::min<std::size_t>(n - first, max_field_reductions));
-            for (unsigned q = 0; q < batch.n; q++) {
-                const std::size_t hi = std::min(rows[first + q], cfg.row_hi);
-                batch.req[q].plane = unsigned(planes_idx[first + q]);
-                batch.req[q].row_lo = unsigned(ghost);
-                batch.req[q].row_hi = unsigned(hi > cfg.row_lo ? ghost + (hi - cfg.row_lo) : ghost);
-                batch.req[q].cols = unsigned(std::min(cols[first + q], cfg.grid_cols));
-            }
-            select_device();
-            reduce_max_abs<Cell>(cfg.device, interior_stream, planes, batch, out + first);
-        }
+        return reduce_max_abs<Cell>(
+            cfg.device, interior_stream, current_planes(),
+            field_requests(extents, cfg.grid_cols, cfg.row_lo, cfg.row_hi, ghost));
     }
 
     /// Copy ONE field of `n_rows` owned rows starting at slab-local row `first_row` into the dense
@@ -372,9 +347,8 @@ template <typename F> class SlabUpdate {
                              std::size_t n_rows) {
         check_row_range(first_row, n_rows);
         join_streams();
-        select_device();
-        copy_plane_rows<Cell>(cfg.device, interior_stream, layout.planes(base, int(epoch & 1)), plane,
-                              ghost + first_row, n_rows, cfg.grid_cols, dst, /*to_device=*/false);
+        copy_plane_rows<Cell>(cfg.device, interior_stream, current_planes(), plane, ghost + first_row,
+                              n_rows, cfg.grid_cols, dst, /*to_device=*/false);
         STST_RT_CHECK(stst_stream_synchronize(interior_stream));
     }
 
@@ -393,19 +367,17 @@ template <typename F> class SlabUpdate {
     void copy_owned_rows_from(PlaneSet const &other_planes, std::size_t other_ghost) {
         join_streams();
         const PlaneSet mine = current_planes();
-        for (std::size_t i = 0; i < Layout::n_planes; i++) {
-            const std::size_t row_bytes = layout.pitch[i] * Layout::plane_bytes(i);
-            STST_RT_CHECK(stst_memcpy_d2d_async(
-                static_cast<unsigned char *>(mine.base[i]) + ghost * row_bytes,
-                static_cast<const unsigned char *>(other_planes.base[i]) + other_ghost * row_bytes,
-                owned_rows() * row_bytes, interior_stream));
-        }
+        auto const &image = layout.image;
+        for (std::size_t i = 0; i < Layout::n_planes; i++)
+            STST_RT_CHECK(stst_memcpy_d2d_async(image.row(mine, i, ghost),
+                                                image.row(other_planes, i, other_ghost),
+                                                owned_rows() * image.row_bytes(i), interior_stream));
         fork_streams();
     }
 
     /**
      * Replace the owned AND the ghost rows by the corresponding rows of a whole grid whose planes
-     * (same row pitch as a slab's: both are "width rounded up to 128 bytes") live on `grid_device` —
+     * (a plane image of the same width, so the same row pitch) live on `grid_device` —
      * one contiguous device-to-device (peer) copy per plane, after `ready` (recorded on the grid's
      * stream) has fired. Because the ghost rows come along, no exchange_halos() is needed; like it,
      * this opens a fresh pair of epochs and is collective: every slab of the grid does it at the same
@@ -431,15 +403,12 @@ template <typename F> class SlabUpdate {
         const std::size_t into = first + ghost - cfg.row_lo; // slab row that holds global row `first`
         if (ready)
             STST_RT_CHECK(stst_stream_wait_event(interior_stream, ready));
-        for (std::size_t i = 0; i < Layout::n_planes; i++) {
-            if (grid_planes.pitch[i] != layout.pitch[i])
-                throw std::logic_error("StencilStream-B200: grid and slab row pitches differ");
-            const std::size_t row_bytes = layout.pitch[i] * Layout::plane_bytes(i);
-            STST_RT_CHECK(stst_memcpy_peer_async(
-                static_cast<unsigned char *>(mine.base[i]) + into * row_bytes, cfg.device,
-                static_cast<const unsigned char *>(grid_planes.base[i]) + first * row_bytes,
-                grid_device, (last - first) * row_bytes, interior_stream));
-        }
+        auto const &image = layout.image;
+        for (std::size_t i = 0; i < Layout::n_planes; i++)
+            STST_RT_CHECK(stst_memcpy_peer_async(image.row(mine, i, into), cfg.device,
+                                                 image.row(grid_planes, i, first), grid_device,
+                                                 (last - first) * image.row_bytes(i),
+                                                 interior_stream));
         // the ghost rows of the new epoch are in place: what the neighbours' flags would say
         for (int s = 0; s < 2; s++) {
             if (has_side(s))
@@ -454,15 +423,11 @@ template <typename F> class SlabUpdate {
     void store_to_grid(PlaneSet const &grid_planes, int grid_device, stst_event_t done) {
         join_streams();
         const PlaneSet mine = current_planes();
-        for (std::size_t i = 0; i < Layout::n_planes; i++) {
-            if (grid_planes.pitch[i] != layout.pitch[i])
-                throw std::logic_error("StencilStream-B200: grid and slab row pitches differ");
-            const std::size_t row_bytes = layout.pitch[i] * Layout::plane_bytes(i);
-            STST_RT_CHECK(stst_memcpy_peer_async(
-                static_cast<unsigned char *>(grid_planes.base[i]) + cfg.row_lo * row_bytes,
-                grid_device, static_cast<const unsigned char *>(mine.base[i]) + ghost * row_bytes,
-                cfg.device, owned_rows() * row_bytes, interior_stream));
-        }
+        auto const &image = layout.image;
+        for (std::size_t i = 0; i < Layout::n_planes; i++)
+            STST_RT_CHECK(stst_memcpy_peer_async(image.row(grid_planes, i, cfg.row_lo), grid_device,
+                                                 image.row(mine, i, ghost), cfg.device,
+                                                 owned_rows() * image.row_bytes(i), interior_stream));
         if (done)
             STST_RT_CHECK(stst_event_record(done, interior_stream));
         fork_streams();
@@ -492,13 +457,11 @@ template <typename F> class SlabUpdate {
             // rows I own next to that neighbour, and where they live in its planes
             const std::size_t my_first = (s == 0) ? ghost : ghost + owned_rows() - ghost;
             const std::size_t their_first = (s == 0) ? ghost + peer.owned_rows : 0;
-            for (std::size_t i = 0; i < Layout::n_planes; i++) {
-                const std::size_t row_bytes = layout.pitch[i] * Layout::plane_bytes(i);
-                STST_RT_CHECK(stst_memcpy_d2d_async(
-                    static_cast<unsigned char *>(theirs.base[i]) + their_first * row_bytes,
-                    static_cast<const unsigned char *>(mine.base[i]) + my_first * row_bytes,
-                    ghost * row_bytes, boundary_stream));
-            }
+            for (std::size_t i = 0; i < Layout::n_planes; i++)
+                STST_RT_CHECK(stst_memcpy_d2d_async(peer.image.row(theirs, i, their_first),
+                                                    layout.image.row(mine, i, my_first),
+                                                    ghost * layout.image.row_bytes(i),
+                                                    boundary_stream));
             raise_flag(s, unsigned(epoch + 1));
         }
         fork_streams();
@@ -560,7 +523,7 @@ template <typename F> class SlabUpdate {
 
     void raise_flag(int s, unsigned value) {
 #if defined(__CUDACC__)
-        select_device();
+        select_device(cfg.device);
         raise_flag_kernel<><<<1, 1, 0, static_cast<cudaStream_t>(boundary_stream)>>>(peer_flag(s),
                                                                                      value);
         if (cudaGetLastError() != cudaSuccess)
@@ -572,18 +535,10 @@ template <typename F> class SlabUpdate {
 #endif
     }
 
-    void select_device() {
-#if defined(__CUDACC__)
-        int current = -1;
-        if (cudaGetDevice(&current) != cudaSuccess || current != cfg.device)
-            cudaSetDevice(cfg.device);
-#endif
-    }
-
     /// boundary stream waits for the interior stream and vice versa
     void join_streams() {
         // Re-recording an event does not disturb waits that were enqueued on its earlier state.
-        select_device();
+        select_device(cfg.device);
         boundary_done->record(boundary_stream);
         STST_RT_CHECK(stst_stream_wait_event(interior_stream, boundary_done->get()));
         interior_done->record(interior_stream);
@@ -600,13 +555,6 @@ template <typename F> class SlabUpdate {
                                  plan.fused_iterations, cfg.tile_rows, pass_through.single_planes());
         if (spec_plan.fused_iterations != plan.fused_iterations)
             throw std::logic_error("StencilStream-B200: pass-through changed the fusion depth");
-    }
-
-    std::size_t plane_set_bytes() const {
-        return layout.plane_offset[1][0] - layout.plane_offset[0][0];
-    }
-    unsigned char *plane_set_begin(int buffer) const {
-        return static_cast<unsigned char *>(base) + layout.plane_offset[buffer][0];
     }
 
     void pass(F const &tf, Cell const &halo_value, std::size_t iteration0, unsigned n_gens,
@@ -729,12 +677,10 @@ template <typename F> class SlabUpdate {
             const std::size_t my_first = (s == 0) ? ghost : owned_rows();        // rows I own there
             const std::size_t ghost_first = (s == 0) ? 0 : ghost + owned_rows(); // rows I receive
             for (std::size_t i = 0; i < Layout::n_planes; i++, n++) {
-                const std::size_t row_bytes = layout.pitch[i] * Layout::plane_bytes(i);
-                unsigned char *plane = static_cast<unsigned char *>(mine.base[i]);
                 peers[n] = nccl_rank[s];
-                send[n] = plane + my_first * row_bytes;
-                recv[n] = plane + ghost_first * row_bytes;
-                send_bytes[n] = recv_bytes[n] = ghost * row_bytes;
+                send[n] = layout.image.row(mine, i, my_first);
+                recv[n] = layout.image.row(mine, i, ghost_first);
+                send_bytes[n] = recv_bytes[n] = ghost * layout.image.row_bytes(i);
             }
         }
         if (n > 0)
@@ -745,59 +691,6 @@ template <typename F> class SlabUpdate {
     void check_row_range(std::size_t first_row, std::size_t n_rows) const {
         if (first_row > owned_rows() || n_rows > owned_rows() - first_row)
             throw std::range_error("StencilStream-B200: row range exceeds the slab");
-    }
-
-    template <bool to_device>
-    void transfer(Cell *cells, std::size_t first_row, std::size_t n_rows) {
-#if defined(__CUDACC__)
-        select_device();
-        const int cur = int(epoch & 1);
-        PlaneSet planes = layout.planes(base, cur);
-        const std::size_t width = cfg.grid_cols;
-        const std::size_t row_bytes = std::max<std::size_t>(width * sizeof(Cell), 1);
-        if (n_rows == 0)
-            return;
-        // pageable host memory moves through the runtime's staging ring, which drains per call:
-        // larger device-side chunks amortise that (see GridStorage::rows_per_chunk)
-        int pinned = 0;
-        (void)stst_host_is_pinned(cells, &pinned);
-        const std::size_t budget = std::size_t(pinned ? 64 : 256) << 20;
-        const std::size_t chunk_rows =
-            std::max<std::size_t>(1, std::min<std::size_t>(n_rows, budget / row_bytes));
-        void *staging[2] = {device_alloc(cfg.device, chunk_rows * width * sizeof(Cell), interior_stream),
-                            device_alloc(cfg.device, chunk_rows * width * sizeof(Cell), interior_stream)};
-        std::size_t chunk = 0;
-        for (std::size_t row = 0; row < n_rows; row += chunk_rows, chunk++) {
-            const std::size_t rows = std::min(chunk_rows, n_rows - row);
-            const std::size_t n = rows * width;
-            Cell *stage = static_cast<Cell *>(staging[chunk & 1]);
-            const unsigned block = 256;
-            const unsigned grid =
-                unsigned(std::min<std::size_t>((n + block - 1) / block, std::size_t(148) * 16));
-            auto s = static_cast<cudaStream_t>(interior_stream);
-            if constexpr (to_device) {
-                STST_RT_CHECK(stst_memcpy_2d_auto(stage, row_bytes, cells + row * width, row_bytes,
-                                                  row_bytes, rows, /*h2d*/ 0, cfg.device,
-                                                  interior_stream));
-                scatter_cells_kernel<Cell><<<grid, block, 0, s>>>(stage, planes, width,
-                                                                  ghost + first_row + row, n);
-            } else {
-                gather_cells_kernel<Cell><<<grid, block, 0, s>>>(stage, planes, width,
-                                                                 ghost + first_row + row, n);
-                STST_RT_CHECK(stst_memcpy_2d_auto(stage, row_bytes, cells + row * width, row_bytes,
-                                                  row_bytes, rows, /*d2h*/ 1, cfg.device,
-                                                  interior_stream));
-            }
-            if (cudaGetLastError() != cudaSuccess)
-                throw std::runtime_error("StencilStream-B200: layout kernel launch failed");
-        }
-        device_free(cfg.device, staging[0], interior_stream);
-        device_free(cfg.device, staging[1], interior_stream);
-#else
-        (void)cells;
-        throw std::runtime_error("StencilStream-B200 must be compiled with nvcc for sm_100a; "
-                                 "there is no CPU fallback");
-#endif
     }
 
     Config cfg;

@@ -2,8 +2,8 @@
  * StencilStream-B200 — the generation loop as sm_100a kernels.
  *
  * This file replaces the device side of the reference's cuda backend: `aos_stencil_kernel`
- * (reference StencilStream/cuda/StencilUpdate.hpp:227-263), `soa_stencil_kernel` (:346-393) and the
- * `scatter_kernel`/`gather_kernel` pair (:294-321, :408-438). The reference launches one sweep per
+ * (reference StencilStream/cuda/StencilUpdate.hpp:227-263) and `soa_stencil_kernel` (:346-393); its
+ * `scatter_kernel`/`gather_kernel` pair lives in PlaneImage.hpp. The reference launches one sweep per
  * (iteration, sub-iteration), one work-item per cell, every work-item gathering its (2r+1)^2
  * neighbourhood from global memory. Here one launch advances the grid by up to
  * `max_fused_iterations` iterations:
@@ -1342,53 +1342,6 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
         run_tile<F, CW, false, (kMode == window_reload ? window_reload : window_shift), kTX, kSpec,
                  true>(tf, halo_value, tdvs, src, dst, no_push, maps, member, smem, &mbar, gy0, gx0,
                        out_lo, out_hi);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// host <-> device layout conversion (array-of-structs staging <-> planes)
-// ------------------------------------------------------------------------------------------------
-
-/**
- * Spread `n_rows` x `width` cells, stored as a dense row-major array of whole cells at `aos`, over the
- * planes, starting at plane row `plane_row0`. Counterpart of the reference's `scatter_kernel`
- * (cuda/StencilUpdate.hpp:294-321), but run once per host->device transfer instead of once per update.
- */
-template <typename Cell>
-__global__ void __launch_bounds__(256)
-    scatter_cells_kernel(const Cell *__restrict__ aos, PlaneSet planes, unsigned long long width,
-                         unsigned long long plane_row0, unsigned long long n_cells) {
-    using L = CellLayout<Cell>;
-    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
-    for (unsigned long long idx = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-         idx < n_cells; idx += stride) {
-        const unsigned long long r = idx / width, c = idx - r * width;
-        const Cell cell = aos[idx];
-        for_each_plane<Cell>([&](auto I) {
-            using T = typename L::template plane_t<I>;
-            static_cast<T *>(planes.base[I])[(plane_row0 + r) * planes.pitch[I] + c] =
-                L::template get<I>(cell);
-        });
-    }
-}
-
-/// Inverse of scatter_cells_kernel; counterpart of the reference's `gather_kernel` (:408-438).
-template <typename Cell>
-__global__ void __launch_bounds__(256)
-    gather_cells_kernel(Cell *__restrict__ aos, PlaneSet planes, unsigned long long width,
-                        unsigned long long plane_row0, unsigned long long n_cells) {
-    using L = CellLayout<Cell>;
-    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
-    for (unsigned long long idx = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-         idx < n_cells; idx += stride) {
-        const unsigned long long r = idx / width, c = idx - r * width;
-        Cell cell;
-        for_each_plane<Cell>([&](auto I) {
-            using T = typename L::template plane_t<I>;
-            L::template get<I>(cell) =
-                static_cast<const T *>(planes.base[I])[(plane_row0 + r) * planes.pitch[I] + c];
-        });
-        aos[idx] = cell;
     }
 }
 
